@@ -22,9 +22,10 @@ Masking belongs to loading a block (run/double_indexed.cpp:122-127, :737-741): r
 made resident (outside the `value` region, like the upload); `e2e` and the reference arm mask inside the timed region.
 
 Reference arm: the stock CLI on the SAME configuration (all queries of rank 0's block, FASTA in, fmt 6 out, whole process wall
-time), `-p` = the fastest of the thread counts tried on a 100 k-query sample; one process run per step, at most --ref-steps steps
-(a full run takes ~10 s).  The cell count of the configuration comes from profiles/workload_cells.json (written by our arm on an
-earlier run, `--emit-cells`): the reference process never loads the CUDA library.
+time), `-p` = the fastest of the thread counts tried on a 100 k-query sample; one process run per step, --steps steps (a full
+run takes ~10 s).  The cell count of the configuration comes from profiles/workload_cells.json, or from the table --cells-json
+names (`--emit-cells` or a run of our arm writes it there; commit the entry to profiles/workload_cells.json to keep it): the
+reference process never loads the CUDA library.
 """
 import argparse, json, os, subprocess, sys, tempfile, threading, time
 
@@ -32,6 +33,8 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 REF_BIN = os.path.join(ROOT, "oracle", "_ref", "diamond")
 CELLS_JSON = os.path.join(ROOT, "profiles", "workload_cells.json")
+DUMP_MAX_ROWS = 1 << 18  # 17 match fields + the row index, float64: 38 MB at most
+DUMP_MAX_TRANSCRIPT = 1 << 22  # edit-transcript bytes of the sampled rows, float32: 16 MB at most
 NO_MASKING = ["--masking", "0", "--motif-masking", "0"]  # parity-ladder rung L1 (SURVEY 8c); [] = the reference's default flags
 
 CONFIGS = {
@@ -51,7 +54,7 @@ CONFIGS = {
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps (at least 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="c2", choices=sorted(CONFIGS))
@@ -60,10 +63,16 @@ def parse():
     ap.add_argument("--sample", type=int, default=100_000, help="queries of the bounded CPU-baseline sample of our arm")
     ap.add_argument("--seed", type=int, default=None)
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    ap.add_argument("--ref-steps", type=int, default=2, help="reference arm: at most this many timed full-configuration runs (and one warm-up)")
-    ap.add_argument("--emit-cells", default=None, help="comma list of reference thread counts: write the configuration's cell counts to gpurun_out/workload_cells.json and exit")
+    ap.add_argument("--emit-cells", default=None, help="comma list of reference thread counts: print the configuration's cell counts (and update --cells-json) and exit")
+    ap.add_argument("--cells-json", default=None, help="cell-count table to read besides profiles/workload_cells.json, and to update with this run's count")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR", help="write the matches of the last timed step as DIR/<field>.npy (float64; "
+                    f"a fixed, seeded sample of at most {DUMP_MAX_ROWS} rows) and their edit transcripts, if any, as DIR/transcripts.npy")
     ap.add_argument("--masking", type=int, default=1, choices=[0, 1], help="1 = reference default flags (tantan + motif masking), 0 = --masking 0 --motif-masking 0 on both arms")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl == "reference" or a.emit_cells):
+        ap.error("--dump-outputs writes what the timed CUDA path computed: not with --impl reference or --emit-cells")
     c = CONFIGS[a.config]
     a.queries = a.queries or c["queries"]; a.db = a.db or c["db"]; a.seed = c["seed"] if a.seed is None else a.seed
     return a
@@ -186,9 +195,9 @@ def cells_key(args, n, threads):
     return f"{args.config}:q{n}:db{args.db}:seed{args.seed}:masking{args.masking}:p{threads}:stream0"
 
 
-def load_cells():
+def load_cells(extra=None):
     best = {}
-    for p in (CELLS_JSON, os.path.join(ROOT, "gpurun_out", "workload_cells.json")):
+    for p in (CELLS_JSON, extra):
         try:
             best.update(json.load(open(p)))
         except Exception:
@@ -199,7 +208,7 @@ def load_cells():
 def lookup_cells(args, n, threads):
     """(cells, note) of the first n queries of rank 0's block; the exact -p entry if there is one, else the entry of another thread
     count of the same configuration (the cell count moves by < 0.1 % with seedp_bits)."""
-    tab = load_cells()
+    tab = load_cells(args.cells_json)
     k = cells_key(args, n, threads)
     if k in tab:
         return tab[k], "cell count of this configuration from profiles/workload_cells.json (our arm, same -p)"
@@ -207,7 +216,38 @@ def lookup_cells(args, n, threads):
     for kk, v in sorted(tab.items()):
         if kk.startswith(pre + ":p"):
             return v, f"cell count from profiles/workload_cells.json entry {kk} (no entry for -p {threads})"
-    return None, "no cached cell count for this configuration: run `python bench.py --emit-cells <threads>` on a GPU box first"
+    return None, ("no cached cell count for this configuration: run `python bench.py --emit-cells <threads> --cells-json FILE` on a B200 "
+                  "and pass the same --cells-json here (or commit the entry to profiles/workload_cells.json)")
+
+
+def sample_matches(m, tr):
+    """The match fields of one step as float64 columns (every integer field is exact there): all rows, or a sorted sample of
+    DUMP_MAX_ROWS row indices drawn with a fixed seed, so that two builds that return the same matches dump the same rows.
+    Where the step returns edit transcripts, those of the sampled rows in row order (up to DUMP_MAX_TRANSCRIPT bytes) stand in for
+    transcript_off: the offsets depend on how the library laid out its transcript buffer (its host thread count), not only on the
+    results."""
+    import numpy as np
+    rows = np.arange(len(m))
+    if len(m) > DUMP_MAX_ROWS:
+        rows = np.sort(np.random.default_rng(0).choice(len(m), DUMP_MAX_ROWS, replace=False))
+    out = {name: m[name][rows].astype(np.float64) for name in m.dtype.names if not name.startswith("_") and name != "transcript_off"}
+    out["row"] = rows.astype(np.float64)
+    out["n_matches"] = np.array([len(m)], dtype=np.float64)
+    if len(tr):
+        parts, total = [], 0
+        for off, n in zip(m["transcript_off"][rows], m["transcript_len"][rows]):
+            if total + int(n) > DUMP_MAX_TRANSCRIPT:
+                break
+            parts.append(tr[int(off): int(off) + int(n)]); total += int(n)
+        out["transcripts"] = (np.concatenate(parts) if parts else np.zeros(0, np.uint8)).astype(np.float32)
+    return out
+
+
+def dump_outputs(d, arrays):
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), a)
 
 
 _result_fd = None
@@ -258,7 +298,7 @@ def main():
                 tried[p] = min(run_reference(args, qs, d, os.path.join(td, "s.tsv"), p) for _ in range(2 if len(cands) > 1 else 1))
             best_p = min(tried, key=tried.get)
             q, d = write_fasta(wl, args.queries, td)
-            warm, steps = min(args.warmup, 1), max(1, min(args.steps, args.ref_steps))
+            warm, steps = min(args.warmup, 1), args.steps
             times = []
             for s in range(warm + steps):
                 dt = run_reference(args, q, d, os.path.join(td, "o.tsv"), best_p)
@@ -283,14 +323,14 @@ def main():
     if args.emit_cells:
         # cell counts of rank 0's block for the given reference thread counts (seedp_bits follows -p), and of the 100 k sample
         wl = make_workload(args, 0)
-        tab = load_cells()
+        tab = load_cells(args.cells_json)
         for p in [int(x) for x in args.emit_cells.split(",")]:
             ctx = api.Context(device=0, threads=p, masking=args.masking, motif_masking=args.masking, **wl["ctx"])
             _, _, st = ctx.blastp(wl["q_raw"], wl["q_lim"], wl["r_raw"], wl["r_lim"])
             ctx.close()
             tab[cells_key(args, args.queries, p)] = st["cells_round1"] + st["cells_round2"]
-        os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
-        json.dump(tab, open(os.path.join(ROOT, "gpurun_out", "workload_cells.json"), "w"), indent=1, sort_keys=True)
+        if args.cells_json:
+            json.dump(tab, open(args.cells_json, "w"), indent=1, sort_keys=True)
         emit(tab)
         return
 
@@ -386,8 +426,9 @@ def main():
     for _ in range(args.warmup):
         step_res()
     c0 = clocks.mark()
-    ms, (m, _, st), tm = timed(step_res, args.steps)
+    ms, (m, tr, st), tm = timed(step_res, args.steps)
     step_ms_res = list(step_ms)
+    dumped = sample_matches(m, tr) if args.dump_outputs and rank == 0 else None
     c1 = clocks.mark()
     clk = clocks.stop(max(c0 - 1, 0), c1 + 1) if rank == 0 else None
     for _ in range(min(args.warmup, 2)):  # the e2e path has its own first-call allocations (block pool, staging)
@@ -478,13 +519,12 @@ def main():
             cpu = {"value": scells / dt / 1e9, "unit": "GCUPS", "cores": ref_threads, "kind": "reference",
                    "sample": f"first {n} queries x full DB, one reference run (FASTA in, fmt 6 out), wall {dt:.2f} s; fmt-6 identical to ours: {same}"}
         # the cell count of this configuration for the reference arm (which must not load the CUDA library)
-        try:
-            tab = load_cells()
+        if args.cells_json:
+            tab = load_cells(args.cells_json)
             tab[cells_key(args, args.queries, ref_threads)] = cells
-            os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
-            json.dump(tab, open(os.path.join(ROOT, "gpurun_out", "workload_cells.json"), "w"), indent=1, sort_keys=True)
-        except Exception:
-            pass
+            json.dump(tab, open(args.cells_json, "w"), indent=1, sort_keys=True)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, dumped)
         out = {"metric": metric, "value": value, "unit": "GCUPS", "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
                "ms_per_step": ms / args.steps, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
                "dtype": "int16 (packed DPX lanes, exact: overflow cascades to the int32 kernels; reference int8/int16 lane semantics)",

@@ -104,7 +104,7 @@ int dmnd_block_broadcast(dmnd_ctx* ctx, int root, dmnd_block* src, dmnd_block** 
 	if (int rc = g_nccl.Broadcast(b->bias, b->bias, padded + 64, NCCL_INT8, root, comm, st)) return nccl_fail("ncclBroadcast(bias)", rc);
 	if (!is_root) {
 		b->has_soft = hdr[2] != 0;
-		++b->content_epoch;
+		b->content_epoch = dmnd_cuda::new_content_epoch();
 		b->h_limits.resize((size_t)nseq + 1);
 		DMND_CUDA_CHECK(cudaMemcpyAsync(b->h_limits.data(), b->limits, sizeof(int64_t) * ((size_t)nseq + 1), cudaMemcpyDeviceToHost, st));
 	}

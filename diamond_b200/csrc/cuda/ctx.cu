@@ -552,6 +552,7 @@ int dmnd_debug_ref_index(dmnd_ctx* ctx, const dmnd_block* ref, int sid, uint64_t
 	DMND_CUDA_CHECK(cudaSetDevice(ctx->device));
 	if (sid < 0 || sid >= ctx->params.n_shapes) { set_error("dmnd_debug_ref_index: bad shape id"); return 1; }
 	dmnd_cuda::RefIndex& ix = ctx->own_index;
+	ctx->own_index_block = nullptr;  // the private index is rebuilt here without a record of its block: the next search rebuilds it again
 	if (dmnd_cuda::build_ref_index(ctx, ref, sid, ix)) return 1;
 	*n = (size_t)ix.nref;
 	if (cap < *n) { set_error("dmnd_debug_ref_index: buffer too small"); return 1; }

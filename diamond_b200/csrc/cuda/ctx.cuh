@@ -2,6 +2,7 @@
 // event-based phase timing.  sm_100a only; no fallback of any kind.
 #pragma once
 #include <cuda_runtime.h>
+#include <atomic>
 #include <cstdint>
 #include <cstdio>
 #include <string>
@@ -69,6 +70,13 @@ struct RefIndex {
 	uint64_t content_epoch = 0, params_hash = 0;  // what the index was built from: the block's content epoch and the context's parameters
 	void release() { keys.release(); locs.release(); bucket.release(); bloom.release(); bitmap.release(); valid = false; }
 };
+
+// Content epochs are unique in the process, not per block: a block allocated where a freed one lived (same address) never
+// matches an index cached for the old one's contents.
+inline uint64_t new_content_epoch() {
+	static std::atomic<uint64_t> next{ 1 };
+	return next.fetch_add(1, std::memory_order_relaxed);
+}
 }  // namespace dmnd_cuda
 
 struct dmnd_block {
@@ -81,7 +89,7 @@ struct dmnd_block {
 	bool has_soft = false;      // dmnd_block_mask(MOTIF) has run: dmnd_search_shape reads `soft`
 	size_t raw_len = 0;
 	uint32_t nseq = 0;
-	uint64_t content_epoch = 1;     // bumped whenever letters or the soft table change (dmnd_block_mask): a cached index of an older epoch is rebuilt
+	uint64_t content_epoch = dmnd_cuda::new_content_epoch();  // renewed whenever letters or the soft table change (dmnd_block_mask): a cached index of an older epoch is rebuilt
 	std::vector<int64_t> h_limits;  // host copy (problem binning needs lengths)
 	std::vector<cudaEvent_t> range_ready;  // dmnd_block_upload_ranges: one event per uploaded sequence range
 	std::vector<uint32_t> range_cuts;      // [nranges + 1] sequence boundaries of those ranges
@@ -120,7 +128,8 @@ struct dmnd_ctx {
 	uint64_t dp_cells_score = 0, dp_cells_trace = 0, dp_cells_padded = 0;  // cells of the problems LAUNCHED (score-only / traceback kernels) and what the register tiles evaluate for them
 	std::vector<dmnd_ctx*> lanes;  // owned lane contexts (dmnd_ctx_lane)
 	dmnd_cuda::RefIndex own_index;  // private reference index when the block carries none
-	const dmnd_block* own_index_block = nullptr;  // ... and the block it was built from (own_index.content_epoch = that block's epoch)
+	const dmnd_block* own_index_block = nullptr;  // ... and the block it was built from (own_index.content_epoch = that block's epoch; the pair
+	                                              // identifies the contents even when a later block reuses the address)
 	dmnd_cuda::DevBuf b_chain_probs;  // dmnd_hits_chain: the DP problems of the device-chained queries (read in place by dmnd_banded_swipe_chained)
 	dmnd_chain_query* chain_q = nullptr; dmnd_dp_problem* chain_probs = nullptr; dmnd_hit* chain_fb_hits = nullptr; dmnd_segment* chain_fb_segs = nullptr; dmnd_hit_site* chain_fb_sites = nullptr;
 	size_t chain_counts[3] = {};

@@ -11,7 +11,7 @@ int block_mask_impl(dmnd_ctx* ctx, dmnd_block* b, int algo, uint32_t s_begin, ui
 	if (algo & ~(DMND_MASK_TANTAN | DMND_MASK_MOTIF)) { set_error("dmnd_block_mask: unknown masking algorithm"); return 1; }
 	cudaStream_t st = ctx->stream;
 	ctx->mask_n = 0;
-	++b->content_epoch;  // letters / soft table change: a seed index cached on the block is stale
+	b->content_epoch = new_content_epoch();  // letters / soft table change: a seed index cached on the block is stale
 	if (n_hard) *n_hard = 0;
 	const size_t p_begin = (size_t)b->h_limits[s_begin], p_end = (size_t)b->h_limits[s_end];
 	const size_t nlet = p_end - p_begin, nseq = s_end - s_begin;

@@ -88,7 +88,7 @@ int effective_cpus() {
 class Pool {
 public:
 	explicit Pool(int n) : n_(n) {
-		for (int t = 1; t < n; ++t) th_.emplace_back([this, t] { loop(t); });
+		for (int t = 1; t < n; ++t) th_.emplace_back([this] { loop(); });
 	}
 	~Pool() {
 		{ std::lock_guard<std::mutex> l(m_); stop_ = true; ++gen_; }
@@ -96,6 +96,10 @@ public:
 		for (auto& t : th_) t.join();
 	}
 	int size() const { return n_; }
+	// Runs f(0) .. f(size() - 1), each once.  Tasks are claimed by whichever thread is free (the caller included) rather than
+	// tied to one worker each: on a host shared with other processes a worker that is descheduled before it starts does not
+	// hold up the call, another thread takes its task.  Callers index their outputs by the task, so results do not depend on
+	// which thread ran it.
 	// Lanes take turns: whoever has host work gets every worker; among waiting lanes the lowest id (the one furthest
 	// along in the staggered pipeline) goes first.
 	void run(const std::function<void(int)>& f, int prio = 0) {
@@ -114,18 +118,35 @@ public:
 		const std::function<void(int)> g(guarded);
 		if (n_ == 1) g(0);
 		else {
-			{ std::lock_guard<std::mutex> l(m_); fn_ = &g; pending_ = n_ - 1; ++gen_; }
+			uint64_t gen;
+			{
+				std::lock_guard<std::mutex> l(m_);
+				fn_ = &g; gen = ++gen_;
+				left_.store(n_, std::memory_order_relaxed);
+				claim_.store(gen << 32, std::memory_order_release);
+			}
 			cv_.notify_all();
-			g(0);
+			work(gen, g);
 			std::unique_lock<std::mutex> l(m_);
-			done_.wait(l, [this] { return pending_ == 0; });
+			done_.wait(l, [this] { return left_.load(std::memory_order_acquire) == 0; });
 		}
 		{ std::lock_guard<std::mutex> l(turn_m_); busy_ = false; }
 		turn_cv_.notify_all();
 		if (first) std::rethrow_exception(first);
 	}
 private:
-	void loop(int t) {
+	// claim_ = (generation << 32) | next task.  A claim only succeeds for the generation the thread read fn_ with, and run() returns
+	// only after every task of its generation has finished, so fn_ is alive whenever a claimed task calls it.
+	void work(uint64_t gen, const std::function<void(int)>& f) {
+		for (;;) {
+			uint64_t c = claim_.load(std::memory_order_acquire);
+			if ((c >> 32) != (gen & 0xffffffffull) || (c & 0xffffffffull) >= (uint64_t)n_) return;
+			if (!claim_.compare_exchange_weak(c, c + 1, std::memory_order_acq_rel)) continue;
+			f((int)(c & 0xffffffffull));
+			if (left_.fetch_sub(1, std::memory_order_acq_rel) == 1) { std::lock_guard<std::mutex> l(m_); done_.notify_one(); }
+		}
+	}
+	void loop() {
 		uint64_t seen = 0;
 		for (;;) {
 			const std::function<void(int)>* f;
@@ -136,8 +157,7 @@ private:
 				if (stop_) return;
 				f = fn_;
 			}
-			(*f)(t);
-			{ std::lock_guard<std::mutex> l(m_); if (--pending_ == 0) done_.notify_one(); }
+			work(seen, *f);
 		}
 	}
 	int n_;
@@ -147,7 +167,8 @@ private:
 	std::vector<int> waiting_;
 	bool busy_ = false;
 	const std::function<void(int)>* fn_ = nullptr;
-	int pending_ = 0;
+	std::atomic<uint64_t> claim_{ 0 };
+	std::atomic<int> left_{ 0 };
 	uint64_t gen_ = 0;
 	bool stop_ = false;
 };

@@ -6,7 +6,7 @@ pipeline over the oracle's K layer."""
 import json, os, subprocess
 import numpy as np
 import pytest
-from conftest import GOLDEN, REF_BIN, ROOT
+from conftest import GOLDEN, ROOT, reference_output, text_digest
 
 CLI = os.path.join(ROOT, "oracle", "_build", "dmnd-oracle-cli")
 XT_FIELDS = "qseqid sseqid pident length mismatch gapopen qstart qend sstart send evalue bitscore cigar btop qseq_gapped sseq_gapped score qlen slen".split()
@@ -106,47 +106,44 @@ def test_blastx_rejects_what_it_does_not_implement(oracle_lib, tmp_path):
     g.close()
 
 
-@pytest.mark.skipif(not os.path.exists(REF_BIN) or not os.path.exists("/root/reference/src/test/SRR14011045_1.fna.gz"), reason="needs the reference build and its test data")
 def test_live_reference_nanopore_reads(oracle_lib, tmp_path):
-    """The reference's own blastx test input (src/test/SRR14011045_1.fna.gz against nr_10k.faa, CMakeLists.txt:544): 200 nanopore
-    reads of 0.3-4 kb full of frame shifts, run here with --fast and the transcript fields."""
+    """The reference's own blastx test input (a sample of src/test/SRR14011045_1.fna.gz against a sample of nr_10k.faa,
+    tests/golden/refdata): nanopore reads of 0.3-4 kb full of frame shifts, run here with --fast and the transcript fields."""
     import gzip
-    q = str(tmp_path / "nano.fna")
-    open(q, "wb").write(gzip.open("/root/reference/src/test/SRR14011045_1.fna.gz").read())
-    d = "/root/reference/src/test/nr_10k.faa"
-    ours, ref = str(tmp_path / "o.tsv"), str(tmp_path / "r.tsv")
-    subprocess.run([REF_BIN, "blastx", "--fast", "-q", q, "-d", d, "-f", "6"] + XT_FIELDS + ["-o", ref, "-p", "8", "--quiet"], capture_output=True, check=True)
+    q, d = str(tmp_path / "nano.fna"), str(tmp_path / "nr.faa")
+    open(q, "wb").write(gzip.open(os.path.join(GOLDEN, "refdata", "SRR14011045_1.fna.gz")).read())
+    open(d, "wb").write(gzip.open(os.path.join(GOLDEN, "refdata", "nr_10k.faa.gz")).read())
+    ours = str(tmp_path / "o.tsv")
+    ref = reference_output("nanopore_reads/fast_transcripts", ["blastx", "--fast", "-q", q, "-d", d, "-f", "6"] + XT_FIELDS + ["-p", "8", "--quiet"])
     r = subprocess.run([CLI, "blastx", "--fast", "-q", q, "-d", d, "-f", "6"] + XT_FIELDS + ["-o", ours, "-p", "8"], capture_output=True, text=True)
     assert r.returncode == 0, r.stderr
-    assert open(ours).read() == open(ref).read() and sum(1 for _ in open(ref)) > 400
+    assert text_digest(open(ours).read()) == ref and ref["lines"] > 20
 
 
-@pytest.mark.skipif(not os.path.exists(REF_BIN), reason="needs the reference build (make ref)")
 @pytest.mark.parametrize("flags", [["--strand", "minus"], ["--strand", "plus", "--min-orf", "30"], ["--query-gencode", "4", "--min-orf", "1"],
                                    ["--unal", "1", "-e", "1e-30"], ["--top", "10"], ["-k", "0", "-c", "1"]])
 def test_blastx_options_like_the_reference(oracle_lib, flags, tmp_path):
     """Translation options (frames of a strand that is not searched stay in the block as X, data/block/block.cpp:95-96; --min-orf
     overrides Config::min_orf_len; NCBI table 4 reads TGA as W), --unal 1 records in nucleotide terms, --top and -k 0: live
-    against the reference on the `bx` reads."""
+    against the reference's output on the `bx` reads."""
     q, d = _files(_bx(), tmp_path)
-    ours, ref = str(tmp_path / "o.tsv"), str(tmp_path / "r.tsv")
+    ours = str(tmp_path / "o.tsv")
     fields = ["-f", "6", "qseqid", "sseqid", "pident", "length", "qstart", "qend", "sstart", "send", "evalue", "bitscore", "qlen", "btop"]
-    subprocess.run([REF_BIN, "blastx", "--fast", "-q", q, "-d", d, "-o", ref, "-p", "8", "--quiet"] + flags + fields, capture_output=True, check=True)
+    ref = reference_output("blastx_options/" + " ".join(flags), ["blastx", "--fast", "-q", q, "-d", d, "-p", "8", "--quiet"] + flags + fields)
     r = subprocess.run([CLI, "blastx", "--fast", "-q", q, "-d", d, "-o", ours, "-p", "8"] + flags + fields, capture_output=True, text=True)
     assert r.returncode == 0, r.stderr
     got = open(ours).read()
-    assert got == open(ref).read() and got.count("\n") > 300
+    assert text_digest(got) == ref and got.count("\n") > 300
     if "--unal" in flags:
         assert sum(l.split("\t")[1] == "*" for l in got.splitlines()) > 50
     if flags[:2] == ["--strand", "minus"]:
         assert all(int(l.split("\t")[4]) > int(l.split("\t")[5]) for l in got.splitlines())  # qstart > qend: reverse strand only
 
 
-@pytest.mark.skipif(not os.path.exists(REF_BIN), reason="needs the reference build (make ref)")
 @pytest.mark.parametrize("mode", ["blastx", "blastp"])
 def test_pairwise_format_translated_and_unaligned(oracle_lib, mode, tmp_path):
     """-f 0 for blastx (" Frame = n" / "-n", query numbering on the read, descending on the reverse strand) and the "No hits found"
-    records of queries that had seed hits but no alignment (strict e-value), live against the reference."""
+    records of queries that had seed hits but no alignment (strict e-value), against the reference's file."""
     from diamond_b200 import synth
     from conftest import workload_blocks
     d = str(tmp_path / "d.faa")
@@ -161,12 +158,12 @@ def test_pairwise_format_translated_and_unaligned(oracle_lib, mode, tmp_path):
         synth.write_fasta(q, w["q_letters"], w["q_off"], "q")
         flags = ["--fast", "-e", "1e-40"]
     synth.write_fasta(d, w["db_letters"], w["db_off"], "d")
-    ours, ref = str(tmp_path / "o.txt"), str(tmp_path / "r.txt")
-    subprocess.run([REF_BIN, mode] + flags + ["-q", q, "-d", d, "-f", "0", "-o", ref, "-p", "8", "--quiet"], capture_output=True, check=True)
+    ours = str(tmp_path / "o.txt")
+    ref = reference_output(f"pairwise_unaligned/{mode}", [mode] + flags + ["-q", q, "-d", d, "-f", "0", "-p", "8", "--quiet"])
     r = subprocess.run([CLI, mode] + flags + ["-q", q, "-d", d, "-f", "0", "-o", ours, "-p", "8"], capture_output=True, text=True)
     assert r.returncode == 0, r.stderr
     got = open(ours).read()
-    assert got == open(ref).read()
+    assert text_digest(got) == ref
     assert got.count("***** No hits found *****") > 20
     if mode == "blastx":
         assert got.count(" Frame = -") > 50 and sum(got.count(f" Frame = {k}\n") for k in (1, 2, 3)) > 50
@@ -272,31 +269,29 @@ def test_frameshift_repeated_calls_on_one_context(oracle_lib):
         assert api.fmt6_translated(m, lens) == outs[k]
 
 
-@pytest.mark.skipif(not os.path.exists(REF_BIN), reason="needs the reference binary (make ref)")
 def test_frameshift_with_reference_blocks_matches_the_reference(oracle_lib, tmp_path):
     """blastx -F 15 -b: per-block legacy runs joined per query; the reference re-derives the statistics of a joined record from its
-    transcript (HspContext::parse), so `length` counts the frameshift marks there -- compared live with the reference."""
+    transcript (HspContext::parse), so `length` counts the frameshift marks there -- compared with the reference's file."""
     q, d = _files(_bx(), tmp_path)
     fields = "qseqid sseqid pident length mismatch gapopen qstart qend sstart send evalue bitscore cigar btop gaps nident qframe".split()
     for flags in (["--fast", "-b0.0002", "-f", "6"] + fields,):  # (--sensitive -b0.0001 -k 5 compared by hand: identical)
-        o1, o2 = str(tmp_path / "ref.tsv"), str(tmp_path / "our.tsv")
-        subprocess.run([REF_BIN, "blastx", "-q", q, "-d", d, "-F", "15", "-p", "8", "--quiet", "-o", o1] + flags, check=True, capture_output=True)
+        o2 = str(tmp_path / "our.tsv")
+        ref = reference_output("frameshift_blocks/" + " ".join(flags[:2]), ["blastx", "-q", q, "-d", d, "-F", "15", "-p", "8", "--quiet"] + flags)
         r = subprocess.run([CLI, "blastx", "-q", q, "-d", d, "-F", "15", "-p", "8", "-o", o2] + flags, capture_output=True, text=True)
         assert r.returncode == 0, r.stderr
-        assert open(o1).read() == open(o2).read()
+        assert text_digest(open(o2).read()) == ref
 
 
-@pytest.mark.skipif(not os.path.exists(REF_BIN), reason="needs the reference binary (make ref)")
 def test_frameshift_score_only_int16_overflow(oracle_lib, tmp_path):
     """A 40 kb read against 32 near-identical 13 500-letter targets: more than -k targets, so the score-only round runs, and every score
     (~79 000) saturates the reference's int16 SIMD lanes -- it repeats such a target alone, in its own band, in int32
-    (dp/swipe/banded_3frame_swipe.cpp:600-607); host/legacy.inc does the same.  Compared live with the reference."""
+    (dp/swipe/banded_3frame_swipe.cpp:600-607); host/legacy.inc does the same.  Compared with the reference's file."""
     from diamond_b200 import synth
     rng = np.random.default_rng(7)
     aa = "ARNDCQEGHILKMFPSTWYV"
     L = 13500
     prot = rng.integers(0, 20, L)
-    q, d, o1, o2 = (str(tmp_path / x) for x in ("q.fna", "d.faa", "ref.tsv", "our.tsv"))
+    q, d, o2 = (str(tmp_path / x) for x in ("q.fna", "d.faa", "our.tsv"))
     open(q, "w").write(">long\n" + "".join(synth._CODONS[aa[a]][0] for a in prot) + "\n")
     with open(d, "w") as f:
         for k in range(32):
@@ -306,8 +301,8 @@ def test_frameshift_score_only_int16_overflow(oracle_lib, tmp_path):
             f.write(f">t{k}\n" + "".join(aa[a] for a in p) + "\n")
         for k in range(200):
             f.write(f">r{k}\n" + "".join(aa[a] for a in rng.integers(0, 20, 300)) + "\n")
-    subprocess.run([REF_BIN, "blastx", "--fast", "-q", q, "-d", d, "-F", "15", "-p", "8", "--quiet", "-o", o1], check=True, capture_output=True)
+    want = reference_output("frameshift_int16_overflow", ["blastx", "--fast", "-q", q, "-d", d, "-F", "15", "-p", "8", "--quiet"])
     r = subprocess.run([CLI, "blastx", "--fast", "-q", q, "-d", d, "-F", "15", "-p", "8", "-o", o2], capture_output=True, text=True)
     assert r.returncode == 0, r.stderr
-    ref = open(o1).read()
-    assert open(o2).read() == ref and len(ref.splitlines()) == 25 and float(ref.splitlines()[0].split("\t")[11]) > 30000  # raw score ~ 79 000 > 65 535
+    got = open(o2).read()
+    assert text_digest(got) == want and len(got.splitlines()) == 25 and float(got.splitlines()[0].split("\t")[11]) > 30000  # raw score ~ 79 000 > 65 535

@@ -1,13 +1,15 @@
 """Masking parity (SURVEY 8f rank 2 -> the reference's DEFAULT flags): tantan hard masking of both blocks
 (masking/tantan.cpp) and motif soft masking (masking/masking.cpp:110-131) in the oracle, pinned against the reference:
  * fmt-6 + --log counters of the L2 goldens (tests/golden/*.l2.*: the reference run with its default flags);
- * the tantan lambda constant against the reference's own LambdaCalculator.cc (compiled here when /root/reference exists);
- * a live default-flag run of the reference on real proteins (src/test/nr_10k.faa, X/B/J letters) when it is present.
+ * the tantan lambda constant against the value the reference's own LambdaCalculator.cc derives (tests/golden/tantan_lambda.txt;
+   compiled from the reference's sources and derived again where DMND_REFERENCE_SRC names a checkout of it);
+ * the reference's default-flag output on real proteins (a sample of its src/test/nr_10k.faa, X/B/J letters), as recorded in
+   tests/golden/reference_outputs.json.
 CPU only."""
 import ctypes as C, json, os, re, subprocess, tempfile
 import numpy as np
 import pytest
-from conftest import GOLDEN, REF_BIN, ROOT, workload_blocks
+from conftest import GOLDEN, ROOT, reference_output, text_digest, workload_blocks
 
 WORKLOADS = ["c1", "fam2", "edge", "long", "rep"]
 
@@ -68,21 +70,17 @@ def test_query_lanes_mask_their_own_ranges(oracle_lib, lanes, monkeypatch):
     assert api.fmt6(m) == open(os.path.join(GOLDEN, "rep.l2.tsv")).read()
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src/lib/tantan"), reason="reference sources not present")
 def test_tantan_lambda_equals_the_reference_lambda_calculator(oracle_lib, tmp_path):
-    """dmnd_params_init hard-codes lambda(BLOSUM62 20x20) = 0x1.4bcf16a672882p-2; re-derive it with the reference's own
-    lib/tantan/LambdaCalculator.cc (compiled from where it lies) and compare the likelihood-ratio table bit for bit."""
+    """dmnd_params_init hard-codes lambda(BLOSUM62 20x20) = 0x1.4bcf16a672882p-2: the value the reference's own
+    lib/tantan/LambdaCalculator.cc derives (tests/golden/tantan_lambda.txt; re-derived from the reference's sources where
+    DMND_REFERENCE_SRC names a checkout of it); the likelihood-ratio table is compared bit for bit."""
     from diamond_b200 import api
-    src = tmp_path / "probe.cpp"
-    src.write_text('#include "LambdaCalculator.hh"\n#include <cstdio>\nint main(){int m[20][20];const int*p[20];for(int i=0;i<20;++i){p[i]=m[i];'
-                   'for(int j=0;j<20;++j)if(scanf("%d",&m[i][j])!=1)return 2;}cbrc::LambdaCalculator lc;lc.calculate(p,20);printf("%a\\n",lc.lambda());return 0;}\n')
-    exe = tmp_path / "probe"
-    subprocess.run(["g++", "-O2", "-I/root/reference/src/lib/tantan", str(src), "/root/reference/src/lib/tantan/LambdaCalculator.cc", "-o", str(exe)], check=True)
     o = api.SearchOpts(); oracle_lib.dmnd_search_opts_default(C.byref(o))
     p = api.Params(); assert oracle_lib.dmnd_params_init(C.byref(o), C.byref(p)) == 0
     s = list(p.score)
-    txt = "\n".join(" ".join(str(s[a * 32 + b]) for b in range(20)) for a in range(20))
-    lam = float.fromhex(subprocess.run([str(exe)], input=txt, capture_output=True, text=True, check=True).stdout.strip())
+    lam = float.fromhex(open(os.path.join(GOLDEN, "tantan_lambda.txt")).read().split()[0])
+    if os.environ.get("DMND_REFERENCE_SRC"):
+        lam = _reference_lambda(os.path.join(os.environ["DMND_REFERENCE_SRC"], "src", "lib", "tantan"), s, tmp_path)
     assert lam == float.fromhex("0x1.4bcf16a672882p-2")
     lr = np.array(list(p.tantan_lr), dtype=np.float32).reshape(32, 32)
     want = np.zeros((32, 32), dtype=np.float32)
@@ -93,36 +91,40 @@ def test_tantan_lambda_equals_the_reference_lambda_calculator(oracle_lib, tmp_pa
     assert o.masking == 1 and o.motif_masking == 1  # the C defaults are the reference's defaults
 
 
-NR10K = "/root/reference/src/test/nr_10k.faa"
+def _reference_lambda(tantan, s, tmp_path):
+    """lambda of the 20x20 part of the score matrix s by the reference's LambdaCalculator, compiled from its sources."""
+    src = tmp_path / "probe.cpp"
+    src.write_text('#include "LambdaCalculator.hh"\n#include <cstdio>\nint main(){int m[20][20];const int*p[20];for(int i=0;i<20;++i){p[i]=m[i];'
+                   'for(int j=0;j<20;++j)if(scanf("%d",&m[i][j])!=1)return 2;}cbrc::LambdaCalculator lc;lc.calculate(p,20);printf("%a\\n",lc.lambda());return 0;}\n')
+    exe = tmp_path / "probe"
+    subprocess.run(["g++", "-O2", "-I" + tantan, str(src), os.path.join(tantan, "LambdaCalculator.cc"), "-o", str(exe)], check=True)
+    txt = "\n".join(" ".join(str(s[a * 32 + b]) for b in range(20)) for a in range(20))
+    return float.fromhex(subprocess.run([str(exe)], input=txt, capture_output=True, text=True, check=True).stdout.strip())
 
 
-@pytest.mark.skipif(not (os.path.exists(REF_BIN) and os.path.exists(NR10K)), reason="reference binary / nr_10k.faa not present")
+NR10K = os.path.join(GOLDEN, "refdata", "nr_10k.faa.gz")  # a sample of the reference's nr_10k.faa
+
+
 def test_live_reference_default_flags_on_real_proteins(tmp_path):
-    """2 000 real proteins (X, B, J letters, long viral polyproteins that are > 50 % motif-covered) against themselves with
+    """Real proteins (X, B, J letters, long viral polyproteins that are > 50 % motif-covered) against themselves with
     the reference's default flags: fmt-6 byte-identical and the --log stage counters equal."""
+    import gzip
     cli = os.path.join(ROOT, "oracle", "_build", "dmnd-oracle-cli")
-    sub = tmp_path / "nr2k.faa"
-    n = 0
-    with open(NR10K) as f, open(sub, "w") as g:
-        for line in f:
-            if line.startswith(">"):
-                n += 1
-                if n > 2000:
-                    break
-            g.write(line)
-    ref_out, our_out = tmp_path / "ref.tsv", tmp_path / "our.tsv"
-    r = subprocess.run([REF_BIN, "blastp", "--fast", "-q", str(sub), "-d", str(sub), "-f", "6", "-o", str(ref_out), "-p", "8", "--log"], capture_output=True, text=True, check=True)
+    sub = tmp_path / "nr.faa"
+    sub.write_bytes(gzip.open(NR10K).read())
+    our_out = tmp_path / "our.tsv"
+    pats = (r"Seeds hit\s+= (\d+)", r"Hits \(filter stage 0\) = (\d+)", r"Hits \(filter stage 1\) = (\d+)", r"Hits \(filter stage 3\) = (\d+)", r"Target hits \(stage 0\) = (\d+)")
+    ref = reference_output("real_proteins/fast", ["blastp", "--fast", "-q", str(sub), "-d", str(sub), "-f", "6", "-p", "8", "--log"], pats)
     o = subprocess.run([cli, "blastp", "--fast", "-q", str(sub), "-d", str(sub), "-o", str(our_out), "-p", "8", "--log"], capture_output=True, text=True, check=True)
-    assert open(ref_out).read() == open(our_out).read() and os.path.getsize(ref_out) > 10000
-    for pat in (r"Seeds hit\s+= (\d+)", r"Hits \(filter stage 0\) = (\d+)", r"Hits \(filter stage 1\) = (\d+)", r"Hits \(filter stage 3\) = (\d+)", r"Target hits \(stage 0\) = (\d+)"):
-        assert re.search(pat, r.stdout + r.stderr).group(1) == re.search(pat, o.stdout + o.stderr).group(1), pat
+    assert text_digest(our_out.read_text(), o.stdout + o.stderr, pats) == ref and ref["bytes"] > 10000
 
 
 def _fasta_blocks(path, limit):
+    import gzip
     from diamond_b200 import api
     alph = {c: i for i, c in enumerate("ARNDCQEGHILKMFPSTWYVBJZX*_")}
     seqs, cur = [], []
-    for line in open(path):
+    for line in gzip.open(path, "rt"):
         if line.startswith(">"):
             if cur:
                 seqs.append("".join(cur)); cur = []
@@ -145,8 +147,6 @@ def test_forward_only_certificate_is_sound(oracle_lib, source):
     computation of the oracle: every sequence below the bound has no masked letter; and the bound is worth having."""
     from diamond_b200 import api, synth
     if source == "nr10k":
-        if not os.path.exists(NR10K):
-            pytest.skip("nr_10k.faa not present")
         raw, lim = _fasta_blocks(NR10K, 4000)
     elif source == "rep":
         raw, lim = workload_blocks("rep")[3:5]
@@ -232,9 +232,10 @@ def test_makedb_and_dmnd_reader(oracle_lib, tmp_path):
     assert r.returncode != 0 and "not permitted" in r.stderr
 
 
-@pytest.mark.skipif(not os.path.exists(REF_BIN), reason="reference binary not present")
 def test_reference_reads_our_database(oracle_lib, tmp_path):
-    """The unmodified reference searches a database written by our makedb and gives the L2 golden."""
+    """The unmodified reference searches a database written by our makedb and gives the L2 golden (its output is stored under
+    the digest of the database file it read: a makedb that writes another file has no stored output)."""
+    import hashlib
     from diamond_b200 import synth
     w, *_ = workload_blocks("edge")
     d, q, o = (str(tmp_path / x) for x in ("d.faa", "q.faa", "o.tsv"))
@@ -242,5 +243,6 @@ def test_reference_reads_our_database(oracle_lib, tmp_path):
     synth.write_fasta(q, w["q_letters"], w["q_off"], "q")
     cli = os.path.join(ROOT, "oracle", "_build", "dmnd-oracle-cli")
     subprocess.run([cli, "makedb", "--in", d, "-d", str(tmp_path / "db")], capture_output=True, check=True)
-    subprocess.run([REF_BIN, "blastp", "--fast", "-q", q, "-d", str(tmp_path / "db.dmnd"), "-f", "6", "-o", o, "-p", "8", "--quiet"], capture_output=True, check=True)
-    assert open(o).read() == open(os.path.join(GOLDEN, "edge.l2.tsv")).read()
+    db = hashlib.sha256(open(tmp_path / "db.dmnd", "rb").read()).hexdigest()
+    ref = reference_output("reads_our_database/" + db, ["blastp", "--fast", "-q", q, "-d", str(tmp_path / "db.dmnd"), "-f", "6", "-p", "8", "--quiet"])
+    assert ref == text_digest(open(os.path.join(GOLDEN, "edge.l2.tsv")).read())

@@ -1,56 +1,47 @@
-"""The reference's OWN regression tests (CMakeLists.txt:534-583, src/test/test.cmake: `diamond ARGS -o NAME.out` must equal the
-committed src/test/NAME.out byte for byte) replayed through this repository's CLI over the oracle-linked host pipeline: every
-case whose options the path implements.  These are the reference's known-answer vectors for the path (SURVEY 8c): real proteins
-(data.faa: 300 sequences; nr_10k.faa), its nanopore reads for blastx (FASTQ and gzipped FASTA), all sensitivity modes from the
-default to --ultra-sensitive, -k / -e / --comp-based-stats 0, the pairwise format.  The command lines are taken from the
-reference's CMakeLists.txt at run time, not retyped here.  CPU only; skipped where /root/reference is absent (the GPU box)."""
-import os, re, shlex, subprocess
+"""The reference's OWN regression tests (its CMakeLists.txt and src/test/test.cmake: `diamond ARGS -o NAME.out` must equal the
+expected NAME.out byte for byte) replayed through this repository's CLI over the oracle-linked host pipeline: every case whose
+options the path implements.  These are the reference's known-answer vectors for the path (SURVEY 8c): real proteins (data.faa:
+300 sequences; a sample of nr_10k.faa), its nanopore reads for blastx (FASTQ and gzipped FASTA), all sensitivity modes from the
+default to --ultra-sensitive, -k / -e / --comp-based-stats 0, the pairwise format.  Inputs and command lines: tests/golden/refdata
+(tests/golden/make_refdata.py); the reference's outputs on them: tests/golden/reference_outputs.json.  The live comparisons
+further down run the reference's CLI on synthetic workloads, recorded the same way.  CPU only."""
+import gzip, json, os, shutil, subprocess
 import pytest
-from conftest import REF_BIN, ROOT, workload_blocks
+from conftest import GOLDEN, ROOT, reference_output, text_digest, workload_blocks
 
-REF = "/root/reference"
-TD = os.path.join(REF, "src", "test")
 CLI = os.path.join(ROOT, "oracle", "_build", "dmnd-oracle-cli")
-# the cases this path covers; the others need options outside it (taxonomy, BLAST databases, DAA, --max-hsps 0, matrix
-# adjustment (--comp-based-stats 2-4), other matrices, --global-ranking, linclust / realign / view)
-CASES = ["blastp", "blastp-mid-sens", "blastp-f0", "blastx-nanopore", "blastx-nanopore-fna",
-         "diamond-test-blastp-default", "diamond-test-blastp-multithreaded", "diamond-test-blastp-more-sensitive",
-         "diamond-test-blastp-very-sensitive", "diamond-test-blastp-ultra-sensitive", "diamond-test-blastp-target-parallel",
-         "diamond-test-blastp-query-indexed", "diamond-test-blastp-comp-based-stats-0", "diamond-test-blastp-target-seqs",
-         "diamond-test-blastp-evalue", "diamond-test-blastp-pairwise-format", "diamond-test-blastp-paf-format", "diamond-test-blastp-top",
-         "blastp-blocked", "diamond-test-blastp-blocked",  # -b: reference blocks + join_blocks
-         "view",        # a DAA file of the reference read back (`view -a test.daa`)
-         "blastp-daa"]  # -f 100: the reference's own archive of 300 x 10 000 proteins, byte for byte (616 KB)
+REFDATA = os.path.join(GOLDEN, "refdata")
+COMMANDS = json.load(open(os.path.join(REFDATA, "ctest_commands.json")))  # {case: argument list with ${TD}}
 
 
-def ctest_commands():
-    """{test name: argument list} from the reference's CMakeLists.txt (add_test(... -DNAME=x "-DARGS=...") and add_diamond_test(x "..."))."""
-    txt = open(os.path.join(REF, "CMakeLists.txt")).read()
-    cmds = {}
-    for m in re.finditer(r'-DNAME=(\S+) "-DARGS=([^"]*)"', txt):
-        cmds[m.group(1)] = m.group(2)
-    for m in re.finditer(r'add_diamond_test\((\S+) "([^"]*)"\)', txt):
-        cmds[m.group(1)] = m.group(2)
-    return {k: shlex.split(v.replace("${TD}", TD)) for k, v in cmds.items()}
+@pytest.fixture(scope="session")
+def td(tmp_path_factory):
+    """The test inputs as the reference's command lines name them (FASTA, FASTQ and DAA files are stored gzip-compressed)."""
+    d = tmp_path_factory.mktemp("refdata")
+    for f in os.listdir(REFDATA):
+        src = os.path.join(REFDATA, f)
+        if f.endswith((".faa.gz", ".fastq.gz", ".daa.gz")):
+            open(d / f[:-3], "wb").write(gzip.open(src).read())
+        else:
+            shutil.copy(src, d / f)
+    return str(d)
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF, "CMakeLists.txt")), reason="needs /root/reference (its test inputs and expected outputs)")
-@pytest.mark.parametrize("name", CASES)
-def test_reference_ctest_case(oracle_lib, name, tmp_path):
-    args = ctest_commands()[name]
+@pytest.mark.parametrize("name", list(COMMANDS))
+def test_reference_ctest_case(oracle_lib, td, name, tmp_path):
+    args = [a.replace("${TD}", td) for a in COMMANDS[name]]
     if "nr_10k.dmnd" in args:  # (the reference's suite builds this database in an earlier test, with taxonomy files that do not enter the search; ours: plain makedb)
         db = str(tmp_path / "nr_10k")
-        subprocess.run([CLI, "makedb", "--in", os.path.join(TD, "nr_10k.faa"), "-d", db], capture_output=True, check=True)
+        subprocess.run([CLI, "makedb", "--in", os.path.join(td, "nr_10k.faa"), "-d", db], capture_output=True, check=True)
         args = [db + ".dmnd" if a == "nr_10k.dmnd" else a for a in args]
     out = str(tmp_path / (name + ".out"))
     r = subprocess.run([CLI] + args + ["-o", out], capture_output=True, text=True)
     assert r.returncode == 0, " ".join(args) + "\n" + r.stderr
-    want = open(os.path.join(TD, name + ".out"), "rb").read()
-    assert open(out, "rb").read() == want, " ".join(args)
-    assert len(want) > 0
+    want = reference_output("ctest/" + name, args)
+    assert text_digest(open(out, "rb").read()) == want, " ".join(args)
+    assert want["bytes"] > 0
 
 
-@pytest.mark.skipif(not os.path.exists(REF_BIN), reason="needs the reference build (make ref)")
 @pytest.mark.parametrize("mode", ["blastp", "blastx"])
 def test_paf_reports_unaligned_queries_like_the_reference(oracle_lib, mode, tmp_path):
     """PAF (Output::Flags::DEFAULT_REPORT_UNALIGNED): a query that had seed hits but no alignment gets the "4 *" record, a query
@@ -70,36 +61,34 @@ def test_paf_reports_unaligned_queries_like_the_reference(oracle_lib, mode, tmp_
         synth.write_dna_fasta(q, w["dna"])
         flags = ["-e", "1e-30"]
     synth.write_fasta(d, w["db_letters"], w["db_off"], "d")
-    ours, ref = str(tmp_path / "o.paf"), str(tmp_path / "r.paf")
-    subprocess.run([REF_BIN, mode] + flags + ["-q", q, "-d", d, "-f", "paf", "-o", ref, "-p", "8", "--quiet"], capture_output=True, check=True)
+    ours = str(tmp_path / "o.paf")
+    ref = reference_output(f"paf_unaligned/{mode}", [mode] + flags + ["-q", q, "-d", d, "-f", "paf", "-p", "8", "--quiet"])
     r = subprocess.run([CLI, mode] + flags + ["-q", q, "-d", d, "-f", "paf", "-o", ours, "-p", "8"], capture_output=True, text=True)
     assert r.returncode == 0, r.stderr
     got = open(ours).read()
-    assert got == open(ref).read()
+    assert text_digest(got) == ref
     lines = got.splitlines()
     assert sum(l.split("\t")[1:3] == ["4", "*"] for l in lines) > 50 and sum(l.split("\t")[4] == "+" for l in lines) > 20
     if mode == "blastx":
         assert sum(l.split("\t")[4] == "-" for l in lines) > 20
 
 
-@pytest.mark.skipif(not os.path.exists(REF_BIN), reason="needs the reference build (make ref)")
 @pytest.mark.parametrize("top,mode", [("50", ["--fast"])])
 def test_top_percent_like_the_reference(oracle_lib, top, mode, tmp_path):
     """--top on protein families (hundreds of targets per query, several ranking chunks): score-ordered culling, the bit-score
     window, one pass of the outer loop (align/culling.cpp:90-141, align/extend.cpp:79-92,336); --top 100 = every target."""
     from diamond_b200 import synth
     w = synth.family_workload(n_fam=3, fam_size=250, n_q=40, seed=77, member_div=(0.02, 0.15), query_div=(0.03, 0.3))
-    q, d, ours, ref = (str(tmp_path / x) for x in ("q.faa", "d.faa", "o.tsv", "r.tsv"))
+    q, d, ours = (str(tmp_path / x) for x in ("q.faa", "d.faa", "o.tsv"))
     synth.write_fasta(q, w["q_letters"], w["q_off"], "q")
     synth.write_fasta(d, w["db_letters"], w["db_off"], "d")
-    subprocess.run([REF_BIN, "blastp"] + mode + ["-q", q, "-d", d, "--top", top, "-o", ref, "-p", "8", "--quiet"], capture_output=True, check=True)
+    ref = reference_output(f"top/{top}", ["blastp"] + mode + ["-q", q, "-d", d, "--top", top, "-p", "8", "--quiet"])
     r = subprocess.run([CLI, "blastp"] + mode + ["-q", q, "-d", d, "--top", top, "-o", ours, "-p", "8"], capture_output=True, text=True)
     assert r.returncode == 0, r.stderr
-    assert open(ours).read() == open(ref).read()
-    assert sum(1 for _ in open(ref)) > 5000
+    assert text_digest(open(ours).read()) == ref
+    assert ref["lines"] > 5000
 
 
-@pytest.mark.skipif(not os.path.exists(REF_BIN), reason="needs the reference build (make ref)")
 @pytest.mark.parametrize("mode", ["blastp", "blastx"])
 def test_sam_format_like_the_reference(oracle_lib, mode, tmp_path):
     """-f sam (output/sam_format.cpp): CIGAR, the aligned query letters, NM / ZI / ZF / ZS and the MD string from the edit transcript,
@@ -117,51 +106,46 @@ def test_sam_format_like_the_reference(oracle_lib, mode, tmp_path):
         q = str(tmp_path / "q.fna")
         synth.write_dna_fasta(q, w["dna"])
     synth.write_fasta(d, w["db_letters"], w["db_off"], "d")
-    ours, ref = str(tmp_path / "o.sam"), str(tmp_path / "r.sam")
+    ours = str(tmp_path / "o.sam")
     flags = ["--fast", "-e", "1e-15", "-q", q, "-d", d, "-f", "sam", "-p", "8"]
-    subprocess.run([REF_BIN, mode] + flags + ["-o", ref, "--quiet"], capture_output=True, check=True)
+    ref = reference_output(f"sam/{mode}", [mode] + flags + ["--quiet"], drop_prefix="@PG")
     r = subprocess.run([CLI, mode] + flags + ["-o", ours], capture_output=True, text=True)
     assert r.returncode == 0, r.stderr
-    a, b = ([l for l in open(p) if not l.startswith("@PG")] for p in (ours, ref))
-    assert a == b and len(a) > 100
+    a = [l for l in open(ours) if not l.startswith("@PG")]
+    assert text_digest("".join(a)) == ref and len(a) > 100
     assert any("^" in l.split("MD:Z:")[1] for l in a if "MD:Z:" in l) or mode == "blastp"
     assert sum(l.split("\t")[1:3] == ["4", "*"] for l in a) > 10
 
 
-@pytest.mark.skipif(not os.path.exists(REF_BIN) or not os.path.exists(os.path.join(TD, "nr_300.faa")), reason="needs the reference build and its test data")
 @pytest.mark.parametrize("mode", ["blastp", "blastx"])
-def test_more_tabular_fields_like_the_reference(oracle_lib, mode, tmp_path):
+def test_more_tabular_fields_like_the_reference(oracle_lib, td, mode, tmp_path):
     """qtitle / stitle (first title of a merged record), positive / ppos, qcovhsp / scovhsp, qframe / qstrand, qseq (the read's nucleotides for blastx) / sseq, with --unal 1, on the
-    reference's real test data (nr_300 proteins / nanopore reads against nr_10k)."""
-    import gzip
+    reference's real test data (samples of the nr_300 proteins / nanopore reads against nr_10k)."""
     fields = "qseqid qtitle sseqid stitle pident positive ppos qcovhsp scovhsp qframe qstrand length evalue qseq sseq".split()
     if mode == "blastp":
-        q = os.path.join(TD, "nr_300.faa")
+        q = os.path.join(td, "nr_300.faa")
     else:
         q = str(tmp_path / "nano.fna")
-        open(q, "wb").write(gzip.open(os.path.join(TD, "SRR14011045_1.fna.gz")).read())
-    flags = ["--fast", "-q", q, "-d", os.path.join(TD, "nr_10k.faa"), "-p", "8", "--unal", "1", "--header", "simple", "-e", "1e-10", "-f", "6"] + fields
-    ours, ref = str(tmp_path / "o.tsv"), str(tmp_path / "r.tsv")
-    subprocess.run([REF_BIN, mode] + flags + ["-o", ref, "--quiet"], capture_output=True, check=True)
+        open(q, "wb").write(gzip.open(os.path.join(td, "SRR14011045_1.fna.gz")).read())
+    flags = ["--fast", "-q", q, "-d", os.path.join(td, "nr_10k.faa"), "-p", "8", "--unal", "1", "--header", "simple", "-e", "1e-10", "-f", "6"] + fields
+    ours = str(tmp_path / "o.tsv")
+    ref = reference_output(f"more_tabular_fields/{mode}", [mode] + flags + ["--quiet"])
     r = subprocess.run([CLI, mode] + flags + ["-o", ours], capture_output=True, text=True)
     assert r.returncode == 0, r.stderr
     got = open(ours).read()
-    assert got == open(ref).read() and got.count("\n") > 300
+    assert text_digest(got) == ref and got.count("\n") > 20
 
 
-@pytest.mark.skipif(not (os.path.exists(REF_BIN) and os.path.exists(TD)), reason="needs the reference build and its test inputs")
 @pytest.mark.parametrize("extra", [["-c1", "-b0.00002"], ["--fast", "-b0.00003", "--top", "10"], ["-b0.00005", "-k", "3", "-f", "6", "qseqid", "sseqid", "evalue", "bitscore", "cigar"]])
-def test_blocked_dmnd_database_matches_reference(oracle_lib, extra, tmp_path):
+def test_blocked_dmnd_database_matches_reference(oracle_lib, td, extra, tmp_path):
     """Reference blocks of a .dmnd database are cut by LETTERS (SequenceFile::load_twopass), FASTA databases by file bytes (the two
     ctest cases above): our -b on a DIAMOND database file against the reference binary, incl. --top (join by score) and transcripts
-    carried through the join."""
+    carried through the join.  The database is written by our makedb, which the reference read for the recording; that our makedb
+    writes the reference's file byte for byte is test_masking.py::test_makedb_and_dmnd_reader."""
     db = str(tmp_path / "db")
-    subprocess.run([REF_BIN, "makedb", "--in", os.path.join(TD, "data.faa"), "-d", db, "--quiet"], check=True, capture_output=True)
-    outs = []
-    for exe in (REF_BIN, CLI):
-        out = str(tmp_path / (os.path.basename(exe) + ".out"))
-        r = subprocess.run([exe, "blastp", "-q", os.path.join(TD, "data.faa"), "-d", db + (".dmnd" if exe == CLI else ""), "-p4", "-o", out] + extra + (["--quiet"] if exe == REF_BIN else []),
-                           capture_output=True, text=True)
-        assert r.returncode == 0, r.stderr
-        outs.append(open(out, "rb").read())
-    assert outs[0] == outs[1] and len(outs[0]) > 1000
+    subprocess.run([CLI, "makedb", "--in", os.path.join(td, "data.faa"), "-d", db], check=True, capture_output=True)
+    ref = reference_output("blocked_dmnd/" + " ".join(extra), ["blastp", "-q", os.path.join(td, "data.faa"), "-d", db, "-p4"] + extra + ["--quiet"])
+    out = str(tmp_path / "o.out")
+    r = subprocess.run([CLI, "blastp", "-q", os.path.join(td, "data.faa"), "-d", db + ".dmnd", "-p4", "-o", out] + extra, capture_output=True, text=True)
+    assert r.returncode == 0, r.stderr
+    assert text_digest(open(out, "rb").read()) == ref and ref["bytes"] > 1000

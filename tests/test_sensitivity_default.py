@@ -5,9 +5,9 @@ S1 goldens (the reference run with no sensitivity flag and its default masking) 
 import ctypes as C, json, os, re, subprocess
 import numpy as np
 import pytest
-from conftest import GOLDEN, REF_BIN, ROOT, workload_blocks
+from conftest import GOLDEN, ROOT, reference_output, text_digest, workload_blocks
 
-NR10K = "/root/reference/src/test/nr_10k.faa"
+NR10K = os.path.join(GOLDEN, "refdata", "nr_10k.faa.gz")  # a sample of the reference's nr_10k.faa
 
 
 @pytest.mark.parametrize("name", ["c1", "fam2", "edge", "long", "rep"])
@@ -108,21 +108,13 @@ def test_ungapped_cutoffs_and_hit_scores(oracle_lib):
     assert (sc == 255).sum() > 100 and (sc > 255).sum() > 0 and (sc < 255).sum() > 100
 
 
-@pytest.mark.skipif(not (os.path.exists(REF_BIN) and os.path.exists(NR10K)), reason="reference binary / nr_10k.faa not present")
 def test_live_reference_default_sensitivity_on_real_proteins(tmp_path):
+    import gzip
     cli = os.path.join(ROOT, "oracle", "_build", "dmnd-oracle-cli")
-    sub = tmp_path / "nr1500.faa"
-    n = 0
-    with open(NR10K) as f, open(sub, "w") as g:
-        for line in f:
-            if line.startswith(">"):
-                n += 1
-                if n > 1500:
-                    break
-            g.write(line)
-    ref_out, our_out = tmp_path / "ref.tsv", tmp_path / "our.tsv"
-    r = subprocess.run([REF_BIN, "blastp", "-q", str(sub), "-d", str(sub), "-f", "6", "-o", str(ref_out), "-p", "8", "--log"], capture_output=True, text=True, check=True)
+    sub = tmp_path / "nr.faa"
+    sub.write_bytes(gzip.open(NR10K).read())
+    our_out = tmp_path / "our.tsv"
+    pats = (r"Seeds hit\s+= (\d+)", r"Hits \(filter stage 0\) = (\d+)", r"Hits \(filter stage 1\) = (\d+)", r"Hits \(filter stage 2\) = (\d+)", r"Hits \(filter stage 3\) = (\d+)")
+    ref = reference_output("real_proteins/default", ["blastp", "-q", str(sub), "-d", str(sub), "-f", "6", "-p", "8", "--log"], pats)
     o = subprocess.run([cli, "blastp", "-q", str(sub), "-d", str(sub), "-o", str(our_out), "-p", "8", "--log"], capture_output=True, text=True, check=True)
-    assert open(ref_out).read() == open(our_out).read() and os.path.getsize(ref_out) > 10000
-    for pat in (r"Seeds hit\s+= (\d+)", r"Hits \(filter stage 0\) = (\d+)", r"Hits \(filter stage 1\) = (\d+)", r"Hits \(filter stage 2\) = (\d+)", r"Hits \(filter stage 3\) = (\d+)"):
-        assert re.search(pat, r.stdout + r.stderr).group(1) == re.search(pat, o.stdout + o.stderr).group(1), pat
+    assert text_digest(our_out.read_text(), o.stdout + o.stderr, pats) == ref and ref["bytes"] > 10000

@@ -1,5 +1,5 @@
 """dmnd_block_broadcast (csrc/cuda/comm.cu): the resident, masked reference block from rank 0 to every rank over NCCL, device to
-device, through the C ABI -- needs two GPUs (skipped on a one-GPU box; run with `gpurun --gpus 2`)."""
+device, through the C ABI -- needs two GPUs (skipped on a machine with one)."""
 import os, subprocess, sys
 import pytest
 from conftest import ROOT
