@@ -103,7 +103,7 @@ FS_RESULT_DTYPE = np.dtype([(n, "<i4") for n in ("score", "q_begin", "q_end", "f
 
 # every symbol include/dmnd_b200.h declares (tests/test_abi.py checks the product library exports them all)
 SYMBOLS = ["dmnd_last_error", "dmnd_set_last_error", "dmnd_backend", "dmnd_ctx_params", "dmnd_create", "dmnd_destroy", "dmnd_ctx_lane", "dmnd_block_upload",
-           "dmnd_block_upload_ranges", "dmnd_block_range_wait", "dmnd_block_compute_bias_range", "dmnd_block_compute_bias_range_async", "dmnd_block_bias_wait", "dmnd_block_free", "dmnd_block_set_bias", "dmnd_block_download_letters", "dmnd_debug_block_soft", "dmnd_debug_ref_index", "dmnd_debug_left_most", "dmnd_block_build_index", "dmnd_block_compute_bias", "dmnd_block_download_bias", "dmnd_block_download_bias_async", "dmnd_copy_wait", "dmnd_host_alloc", "dmnd_host_free", "dmnd_hits_xdrop", "dmnd_hits_xdrop_sites", "dmnd_block_clear_seed_mask", "dmnd_block_clear_seed_mask_range", "dmnd_block_mask", "dmnd_block_mask_fetch", "dmnd_hits_gapped_filter", "dmnd_comm_unique_id", "dmnd_comm_init", "dmnd_comm_destroy", "dmnd_block_broadcast", "dmnd_block_alloc_empty", "dmnd_block_geometry", "dmnd_block_download_limits", "dmnd_hits_chain", "dmnd_hits_chain_fetch", "dmnd_banded_swipe_chained",
+           "dmnd_block_upload_ranges", "dmnd_block_range_wait", "dmnd_block_compute_bias_range", "dmnd_block_free", "dmnd_block_set_bias", "dmnd_block_download_letters", "dmnd_debug_block_soft", "dmnd_debug_ref_index", "dmnd_debug_left_most", "dmnd_block_build_index", "dmnd_block_compute_bias", "dmnd_block_download_bias", "dmnd_block_download_bias_async", "dmnd_copy_wait", "dmnd_host_alloc", "dmnd_host_free", "dmnd_hits_xdrop", "dmnd_hits_xdrop_sites", "dmnd_block_clear_seed_mask", "dmnd_block_clear_seed_mask_range", "dmnd_block_mask", "dmnd_block_mask_fetch", "dmnd_hits_gapped_filter", "dmnd_comm_unique_id", "dmnd_comm_init", "dmnd_comm_destroy", "dmnd_block_broadcast", "dmnd_block_alloc_empty", "dmnd_block_geometry", "dmnd_block_download_limits", "dmnd_hits_chain", "dmnd_hits_chain_fetch", "dmnd_banded_swipe_chained",
            "dmnd_search_shape", "dmnd_search_shape_range", "dmnd_hits_count", "dmnd_hits_download", "dmnd_hits_free", "dmnd_banded_swipe", "dmnd_banded_3frame_swipe",
            "dmnd_timing_fetch", "dmnd_measure_int_peak", "dmnd_measure_int_peak_packed", "dmnd_search_opts_default", "dmnd_mode_motif_masking", "dmnd_alignment_stats", "dmnd_params_init", "dmnd_blastp", "dmnd_blastp_resident",
            "dmnd_result_matches", "dmnd_result_transcripts", "dmnd_result_stats", "dmnd_result_masked_positions", "dmnd_result_unaligned", "dmnd_result_free"]

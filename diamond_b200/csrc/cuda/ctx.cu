@@ -440,34 +440,6 @@ int dmnd_block_compute_bias_range(dmnd_ctx* ctx, dmnd_block* b, int mode, uint32
 	return 0;
 }
 
-int dmnd_block_compute_bias_range_async(dmnd_ctx* ctx, dmnd_block* b, int mode, uint32_t s_begin, uint32_t s_end) {
-	DMND_CUDA_CHECK(cudaSetDevice(ctx->device));
-	if (mode != 0 && mode != 1) { set_error("dmnd_block_compute_bias: unknown mode"); return 1; }
-	if (s_begin > s_end || s_end > b->nseq) { set_error("dmnd_block_compute_bias_range: sequence range out of bounds"); return 1; }
-	if (s_begin == s_end) return 0;
-	if (!ctx->ev_bias) DMND_CUDA_CHECK(cudaEventCreateWithFlags(&ctx->ev_bias, cudaEventDisableTiming));
-	// behind everything this context has issued (the range may just have been masked), beside everything it issues next
-	DMND_CUDA_CHECK(cudaEventRecord(ctx->ev_bias, ctx->stream));
-	DMND_CUDA_CHECK(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_bias, 0));
-	const size_t lo = (size_t)b->h_limits[s_begin], hi = (size_t)b->h_limits[s_end];
-	DMND_CUDA_CHECK(cudaMemsetAsync(b->bias + lo, 0, hi - lo, ctx->copy_stream));
-	if (mode == 1) {
-		const uint32_t n = s_end - s_begin;
-		hauser_kernel<<<(n + 127) / 128, 128, 0, ctx->copy_stream>>>(b->letters, b->limits + s_begin, n, ctx->d_params, b->bias);
-		++ctx->launches;
-		DMND_CUDA_CHECK(cudaGetLastError());
-	}
-	DMND_CUDA_CHECK(cudaEventRecord(ctx->ev_bias, ctx->copy_stream));
-	ctx->bias_pending = true;
-	return 0;
-}
-
-int dmnd_block_bias_wait(dmnd_ctx* ctx) {
-	DMND_CUDA_CHECK(cudaSetDevice(ctx->device));
-	if (ctx->bias_pending) { DMND_CUDA_CHECK(cudaStreamWaitEvent(ctx->stream, ctx->ev_bias, 0)); ctx->bias_pending = false; }
-	return 0;
-}
-
 int dmnd_block_compute_bias(dmnd_ctx* ctx, dmnd_block* b, int mode) {
 	DMND_CUDA_CHECK(cudaSetDevice(ctx->device));
 	if (mode != 0 && mode != 1) { set_error("dmnd_block_compute_bias: unknown mode"); return 1; }

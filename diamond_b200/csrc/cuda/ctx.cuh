@@ -108,8 +108,7 @@ struct dmnd_ctx {
 	uint8_t* d_matcher[DMND_MAX_SHAPES + 1] = {};  // PatternMatcher tables
 	uint32_t matcher_minlen[DMND_MAX_SHAPES + 1] = {}, matcher_suffix[DMND_MAX_SHAPES + 1] = {};
 	cudaStream_t stream = nullptr, copy_stream = nullptr;
-	cudaEvent_t ev_copy = nullptr, ev_bias = nullptr;  // ev_bias: end of the last dmnd_block_compute_bias_range_async on copy_stream
-	bool bias_pending = false;
+	cudaEvent_t ev_copy = nullptr;
 	int sm_count = 148;
 	// scratch
 	dmnd_cuda::DevBuf b_keys, b_keys2, b_vals, b_vals2, b_cub, b_bucket, b_entries, b_pairs, b_hits, b_hits2, b_counters;

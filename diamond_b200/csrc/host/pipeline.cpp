@@ -318,6 +318,10 @@ struct Env {
 	bool report_cutoff(int score, double evalue) const { return min_bit_score != 0.0 ? sc->bitscore(score) >= min_bit_score : evalue <= max_evalue; }
 	bool hauser, want_transcript;
 	bool fuse;  // see Driver::start
+	// The bridge from hits to DP problems runs on the device (dmnd_hits_chain) for single-shape blastp without a gapped filter: the hits
+	// never come to the host, the round-1 problem list of every query with <= 64 targets is produced and aligned in HBM, and only
+	// queries with ranking chunks (or pairs beyond the device code's capacities) take the host code.
+	bool bridge = false;
 	// --id / --query-cover / --subject-cover (config.min_id, query_cover, subject_cover): with any of them set the reference only SORTS the
 	// targets after round 1 (first_round_culling = !have_filters || --top, align/extend.cpp:94-96,288) and runs round 2 in steps
 	double min_id = 0.0, query_cover = 0.0, subject_cover = 0.0, approx_min_id = 0.0;
@@ -450,6 +454,11 @@ struct Workspace {
 	HostBuf<dmnd_hit_site> sitev;
 	struct HitSeg { dmnd_hit h; dmnd_segment s; dmnd_hit_site site; uint8_t gf; };
 	std::vector<HitSeg> hs;
+	// hits [b, e) of hv / segv / sitev / gfv as the records load_hits and legacy_init take (built in place in hs)
+	HitSeg* gather(size_t b, size_t e) {
+		for (size_t x = b; x < e; ++x) hs[x] = HitSeg{ hv[x], segv[x], sitev[x], gfv[x] };
+		return hs.data() + b;
+	}
 	std::vector<size_t> qstart;
 	std::vector<QueryState> qs;
 	HostBuf<dmnd_dp_problem> p1, p2, cprobs;  // cprobs / cres / cq: dmnd_hits_chain's problem list, its results, its per-query records
@@ -458,7 +467,8 @@ struct Workspace {
 	HostBuf<uint8_t> tr;
 	RawBuf<dmnd_match> out_matches;   // lane output when several lanes run (copied into the result afterwards)
 	RawBuf<uint8_t> out_transcripts;
-	std::vector<dmnd_hit> acc_hits; std::vector<dmnd_segment> acc_segs; std::vector<dmnd_hit_site> acc_sites; std::vector<uint8_t> acc_gf, gf_tmp, gfv;  // hits of all shapes (several shapes only)
+	std::vector<dmnd_hit> acc_hits; std::vector<dmnd_segment> acc_segs; std::vector<dmnd_hit_site> acc_sites; std::vector<uint8_t> acc_gf;  // hits of all shapes (several shapes only)
+	std::vector<uint8_t> gfv;         // per hit of hv: passes the gapped filter (1 where the mode has none)
 	std::vector<uint64_t> mask_pos;   // letters of this lane's query range that dmnd_block_mask turned into X
 	PatchSet q_patch;
 };
@@ -891,6 +901,13 @@ void Driver::finish_outer(QueryState& q) {
 	q.phase = PH_DONE;
 }
 
+// Transcript bytes the traceback kernel may need for problems p[0, n): qlen + tlen per problem.
+static size_t transcript_cap(const Env& e, const dmnd_dp_problem* p, size_t n) {
+	size_t cap = 0;
+	for (size_t k = 0; k < n; ++k) cap += (size_t)e.qlen(p[k].query) + (size_t)e.tlen(p[k].target);
+	return cap;
+}
+
 int Driver::run_waves() {
 	Workspace& w = *ws;
 	Prof prof;
@@ -932,7 +949,7 @@ int Driver::run_waves() {
 		if (!w.p2.empty()) {
 			size_t cap = 0;
 			if (env.want_transcript) {
-				for (const dmnd_dp_problem& pr : w.p2) cap += (size_t)env.qlen(pr.query) + (size_t)env.tlen(pr.target);
+				cap = transcript_cap(env, w.p2.data(), w.p2.size());
 				if (w.tr.resize(ctx, cap)) return 1;
 				trp = w.tr.data();
 			}
@@ -1163,234 +1180,121 @@ struct SeedTurn {
 	void pass(int lane) { { std::lock_guard<std::mutex> l(m); turn = std::max(turn, lane + 1); } cv.notify_all(); }
 };
 
-// Block mode of the device-bridged path (one shape, one context, no gapped filter): the seed stage and dmnd_hits_chain run ONCE over the
-// whole query block (lane 0, after every lane has prepared -- waited for, masked, biased -- its own query range), then every lane takes the
-// queries of its range from the shared chain records: banded swipe on the lane's context (at most two calls in flight, in lane order) and the
-// host work beside the next lane's kernels.  The idea: a seed stage per lane costs 38 ms of wall time per 10^6 queries for 19 ms of kernels
-// (the lanes' seed kernels queue behind each other's DP), one seed stage over the block takes 15 ms.  Measured on a B200 (same box, 10 steps
-// each, profiles/ab_block_mode_r2.txt): 55.0 ms per resident step and 80.8 ms end to end against 50.2 / 75.3 ms for the per-lane pipeline --
-// the block's seed stage runs alone on the GPU, and what the lanes lose in queueing they win back in overlap.  Kept behind
-// DMND_PIPELINE_BLOCK=1 (results are identical: the CPU suite runs both forms); the per-lane pipeline is the default.
-struct BlockStage {
-	bool on = false;
-	int nlanes = 0;
-	std::mutex m;
-	std::condition_variable cv;
-	int prepped = 0;      // lanes whose query range is resident, masked and biased
-	int state = 0;        // 0 = chain records not there yet, 1 = published, -1 = failed
-	Workspace* root = nullptr;  // lane 0's workspace: cq / cprobs / hv / segv / sitev of the whole block
-	dmnd_chain_out co{};
-	int dp_started = 0, dp_done = 0;
-	void arrive() { { std::lock_guard<std::mutex> l(m); ++prepped; } cv.notify_all(); }
-	void wait_all_prepped() { std::unique_lock<std::mutex> l(m); cv.wait(l, [&] { return prepped >= nlanes || state < 0; }); }
-	void publish(int st) { { std::lock_guard<std::mutex> l(m); if (state == 0) state = st; } cv.notify_all(); }
-	int wait_published() { std::unique_lock<std::mutex> l(m); cv.wait(l, [&] { return state != 0; }); return state; }
-	void dp_begin(int lane) { std::unique_lock<std::mutex> l(m); cv.wait(l, [&] { return state < 0 || (dp_started >= lane && dp_done >= lane - 1); }); dp_started = std::max(dp_started, lane + 1); cv.notify_all(); }
-	void dp_end(int lane) { { std::lock_guard<std::mutex> l(m); dp_started = std::max(dp_started, lane + 1); dp_done = std::max(dp_done, lane + 1); } cv.notify_all(); }
-	void abort() { { std::lock_guard<std::mutex> l(m); state = -1; prepped = nlanes; dp_started = dp_done = nlanes; } cv.notify_all(); }
+// However a lane leaves (error or exception), the lanes behind it must not wait for its masking or its seed turn.
+struct TurnRelease { SeedTurn& turn; int lane; ~TurnRelease() { turn.set_masked(lane); turn.pass(lane); } };
+
+struct HitsGuard {  // the hits of one search, freed on every way out of the scope that searched
+	dmnd_ctx* ctx; dmnd_hits* h = nullptr;
+	explicit HitsGuard(dmnd_ctx* c) : ctx(c) {}
+	HitsGuard(const HitsGuard&) = delete;
+	~HitsGuard() { dmnd_hits_free(ctx, h); }
 };
 
-static int lane_run(dmnd_ctx* ctx, dmnd_block* qb, const dmnd_block* rb, const Env& env, const Scoring& sc, uint32_t q_begin, uint32_t q_end,
-                    Workspace& w, int host_threads, LaneOut& lo, int lane, SeedTurn& seed_turn, BlockStage& bs) {
-	auto t_total = Clock::now();
-	Driver d;
-	d.ctx = ctx; d.qb = qb; d.rb = rb; d.ws = &w; d.T = host_threads; d.env = env;
-	std::memset(&d.stats, 0, sizeof d.stats);
-	dmnd_timing tm0; dmnd_timing_fetch(ctx, &tm0, DMND_TIMING_THIS_CONTEXT);  // snapshot: the device counters of this call are reported as a delta
+static void add_counters(dmnd_stage_counters& a, const dmnd_stage_counters& b) {
+	a.seeds_hit += b.seeds_hit; a.seed_hits += b.seed_hits; a.tentative_matches1 += b.tentative_matches1;
+	a.tentative_matches2 += b.tentative_matches2; a.tentative_matches3 += b.tentative_matches3; a.masked_seeds += b.masked_seeds;
+}
 
-	// ---- seed stage (run_ref_chunk: one search_shape per shape; FAST has one shape)
-	Prof prof;
-	auto t0 = Clock::now();
-	dmnd_hits* hits = nullptr;
-	w.lane = lane;
-	// this lane's query range may still be on its way (dmnd_block_upload_ranges); its composition bias is computed here, on
-	// the lane's stream, as soon as the letters are there
-	int prep_rc = dmnd_block_range_wait(ctx, qb, q_begin, q_end);
-	if (!prep_rc && env.mask_algo) {
-		// "Masking queries" (run/double_indexed.cpp:737-741) + the query block's motif table, for this lane's range; the host
-		// only learns WHICH letters became X and patches private copies of those sequences
+// The device time, launch and byte counters between two snapshots of a context's timing (the DP cell counters stay 0).
+static dmnd_timing device_delta(const dmnd_timing& t1, const dmnd_timing& t0) {
+	dmnd_timing d{};
+	d.seed_ms = t1.seed_ms - t0.seed_ms; d.dp_score_ms = t1.dp_score_ms - t0.dp_score_ms; d.dp_trace_ms = t1.dp_trace_ms - t0.dp_trace_ms;
+	d.h2d_ms = t1.h2d_ms - t0.h2d_ms; d.d2h_ms = t1.d2h_ms - t0.d2h_ms;
+	d.launches = t1.launches - t0.launches; d.h2d_bytes = t1.h2d_bytes - t0.h2d_bytes; d.d2h_bytes = t1.d2h_bytes - t0.d2h_bytes;
+	return d;
+}
+
+// Waits for the lane's query range (dmnd_block_upload_ranges), masks it ("Masking queries", run/double_indexed.cpp:737-741, + the query
+// block's motif table: the host only learns WHICH letters became X and patches private copies of those sequences), computes its
+// composition bias, then waits for the next lane's masking and for this lane's seed turn.
+static int prepare_range(Driver& d, uint32_t q_begin, uint32_t q_end, int lane, SeedTurn& turn, Prof& prof) {
+	Workspace& w = *d.ws;
+	const Env& env = d.env;
+	int rc = dmnd_block_range_wait(d.ctx, d.qb, q_begin, q_end);
+	if (!rc && env.mask_algo) {
 		uint64_t n_hard = 0;
-		prep_rc = dmnd_block_mask(ctx, qb, env.mask_algo, q_begin, q_end, &n_hard);
+		rc = dmnd_block_mask(d.ctx, d.qb, env.mask_algo, q_begin, q_end, &n_hard);
 		w.mask_pos.resize((size_t)n_hard);
-		if (!prep_rc && n_hard) prep_rc = dmnd_block_mask_fetch(ctx, w.mask_pos.data(), w.mask_pos.size());
-		if (!prep_rc) { w.q_patch.build(env.q_letters, env.q_limits, env.nq, q_begin, q_end, w.mask_pos.data(), w.mask_pos.size()); d.env.q_patch = &w.q_patch; }
+		if (!rc && n_hard) rc = dmnd_block_mask_fetch(d.ctx, w.mask_pos.data(), w.mask_pos.size());
+		if (!rc) { w.q_patch.build(env.q_letters, env.q_limits, env.nq, q_begin, q_end, w.mask_pos.data(), w.mask_pos.size()); d.env.q_patch = &w.q_patch; }
 	}
-	seed_turn.set_masked(lane);  // (dmnd_block_mask returns when the range is masked on the device; also set on failure so nobody waits forever)
-	// the composition bias of this range.  DMND_ASYNC_BIAS=1 computes it on the lane's second stream beside the seed stage (which reads
-	// letters only; the first consumers wait on the device, dmnd_block_bias_wait below): it removes a 2 ms bubble at the start of a step
-	// but two of two B200 runs with it showed a 190 ms outlier step, so the synchronous form stays the default (profiles/ab_seed_r2.txt)
-	// (block mode: lane 0 extends the hits of EVERY range, so each lane's bias must be complete when the lane reports in)
-	prep_rc = prep_rc || ((getenv("DMND_ASYNC_BIAS") && !bs.on) ? dmnd_block_compute_bias_range_async(ctx, qb, env.hauser ? 1 : 0, q_begin, q_end) : dmnd_block_compute_bias_range(ctx, qb, env.hauser ? 1 : 0, q_begin, q_end));
-	if (!bs.on) seed_turn.wait_masked(lane + 1);  // (block mode: lane 0 searches the whole block after EVERY lane has prepared its range)
-	prof.lane = lane;
+	turn.set_masked(lane);  // (dmnd_block_mask returns when the range is masked on the device; also set on failure so nobody waits forever)
+	rc = rc || dmnd_block_compute_bias_range(d.ctx, d.qb, env.hauser ? 1 : 0, q_begin, q_end);
+	turn.wait_masked(lane + 1);
 	prof.lap("wait, mask, bias");
-	if (!bs.on) seed_turn.wait_for(lane);
+	turn.wait_for(lane);
 	prof.lap("wait for the seed turn");
+	return rc;
+}
+
+// Seed stage of the bridged mode (Env::bridge): the search, then dmnd_hits_chain turns the hits into the round-1 problem list on the
+// device.  Only the per-query records, the problems and the hits of DMND_CHAIN_HOST queries come back.
+static int seed_bridged(Driver& d, uint32_t q_begin, uint32_t q_end, int lane, SeedTurn& turn, Clock::time_point t0, dmnd_chain_out& co, Prof& prof) {
+	Workspace& w = *d.ws;
+	HitsGuard hits(d.ctx);
+	const int rc = dmnd_search_shape_range(d.ctx, d.qb, d.rb, 0, q_begin, q_end, &hits.h, &d.stats.seed);
+	turn.pass(lane);
+	if (rc) return 1;
+	prof.lap("search_shape");
+	d.stats.hits = dmnd_hits_count(hits.h);
+	d.stats.seed_ms = ms_since(t0);
+	t0 = Clock::now();
+	if (dmnd_hits_chain(d.ctx, d.qb, d.rb, hits.h, d.env.sc->raw_ungapped_xdrop, d.env.band_slow ? 1 : 0, 64, &co)) return 1;
+	const size_t nh = (size_t)co.n_host_hits;
+	if (w.cq.resize(d.ctx, (size_t)co.n_queries) || w.cprobs.resize(d.ctx, (size_t)co.n_problems) || w.cres.resize(d.ctx, (size_t)co.n_problems)
+	    || w.hv.resize(d.ctx, nh) || w.segv.resize(d.ctx, nh) || w.sitev.resize(d.ctx, nh))
+		return 1;
+	if (dmnd_hits_chain_fetch(d.ctx, w.cq.data(), w.cprobs.data(), w.hv.data(), w.segv.data(), w.sitev.data())) return 1;
+	d.stats.host_bridge_ms += ms_since(t0);
+	prof.lap("hits_chain (device bridge)");
+	w.gfv.assign(nh, 1);  // (the mode has no gapped filter)
+	return 0;
+}
+
+// Seed stage of every other mode, run_ref_chunk's loop over the shapes (run/double_indexed.cpp:185-214): SEED_MASK bits set by one shape
+// stay visible to the next ones.  Every hit comes with its x-drop segment (align/ungapped.cpp:88), its site in the reference block and,
+// where the mode has one, its gapped-filter verdict.  The hits of all shapes feed one extension: the shapes' query-grouped lists are
+// merged into one (counting sort by query, stable).  Leaves the lane's hits in hv / segv / sitev / gfv [0, nh).
+static int seed_host(Driver& d, uint32_t q_begin, uint32_t q_end, int lane, SeedTurn& turn, size_t& nh, Prof& prof) {
+	Workspace& w = *d.ws;
+	const Env& env = d.env;
 	const int n_shapes = env.n_shapes;
-	size_t nh = 0;
-	// The bridge from hits to DP problems runs on the device (dmnd_hits_chain) for single-shape blastp without a gapped filter:
-	// the hits never come to the host, the round-1 problem list of every query with <= 64 targets is produced and aligned in HBM,
-	// and only queries with ranking chunks (or pairs beyond the device code's capacities) take the host code below.
-	const bool bridge = n_shapes == 1 && env.fuse && env.contexts == 1 && !env.gapped_filter && !env.frame_shift && getenv("DMND_HOST_BRIDGE") == nullptr;
-	dmnd_chain_out co;
-	std::memset(&co, 0, sizeof co);
-	// block mode: this lane's slice of the shared chain records -- queries [bk0, bk1) of bs.root->cq, their problems [bp0, bp1) of
-	// bs.root->cprobs, and (queries that take the host path) their hits [bh0, bh1) of bs.root->hv / segv / sitev
-	size_t bk0 = 0, bk1 = 0, bp0 = 0, bp1 = 0, bh0 = 0, bh1 = 0;
-	if (bs.on && bridge) {
-		struct DpGuard { BlockStage& b; int lane; bool armed = true; ~DpGuard() { if (armed) b.dp_end(lane); } } dp_guard{ bs, lane };  // a lane that leaves early must not block the DP order
-		bs.arrive();
-		if (lane == 0) {
-			Workspace& rw = w;
-			bs.root = &rw;
-			bs.wait_all_prepped();
-			int rc = prep_rc || bs.state < 0;
-			if (!rc) rc = dmnd_search_shape_range(ctx, qb, rb, 0, 0, env.nq, &hits, &d.stats.seed);
-			prof.lap("search_shape (whole block)");
-			if (!rc) {
-				d.stats.hits = dmnd_hits_count(hits);
-				d.stats.seed_ms = ms_since(t0);
-				t0 = Clock::now();
-				rc = dmnd_block_bias_wait(ctx) || dmnd_hits_chain(ctx, qb, rb, hits, sc.raw_ungapped_xdrop, env.band_slow ? 1 : 0, 64, &bs.co);
-				dmnd_hits_free(ctx, hits);
-				const size_t hn = (size_t)bs.co.n_host_hits;
-				rc = rc || rw.cq.resize(ctx, (size_t)bs.co.n_queries) || rw.cprobs.resize(ctx, (size_t)bs.co.n_problems) || rw.hv.resize(ctx, hn) || rw.segv.resize(ctx, hn) || rw.sitev.resize(ctx, hn);
-				rc = rc || dmnd_hits_chain_fetch(ctx, rw.cq.data(), rw.cprobs.data(), rw.hv.data(), rw.segv.data(), rw.sitev.data());
-				rc = rc || dmnd_block_clear_seed_mask_range(ctx, qb, 0, env.nq);  // run/double_indexed.cpp:211-212
-				d.stats.host_bridge_ms += ms_since(t0);
-				prof.lap("hits_chain (whole block)");
-			}
-			bs.publish(rc ? -1 : 1);
-			if (rc) return 1;
-		}
-		else if (bs.wait_published() < 0 || prep_rc) { if (!prep_rc) dmnd_set_last_error("dmnd_blastp: the block's seed stage failed (lane 0 carries the message)"); return 1; }
-		if (lane != 0 && dmnd_block_bias_wait(ctx)) return 1;
-		t0 = Clock::now();
-		const Workspace& rw = *bs.root;
-		co = bs.co;
-		const dmnd_chain_query* cqa = rw.cq.data();
-		const size_t nqa = (size_t)co.n_queries;
-		bk0 = (size_t)(std::lower_bound(cqa, cqa + nqa, q_begin, [](const dmnd_chain_query& c, uint32_t q) { return c.query < q; }) - cqa);
-		bk1 = (size_t)(std::lower_bound(cqa, cqa + nqa, q_end, [](const dmnd_chain_query& c, uint32_t q) { return c.query < q; }) - cqa);
-		bool pset = false, hset = false;
-		for (size_t k = bk0; k < bk1; ++k) {
-			const dmnd_chain_query& c = cqa[k];
-			if (c.flags & DMND_CHAIN_HOST) { if (!hset) { bh0 = c.first; hset = true; } bh1 = (size_t)c.first + c.n_hits; }
-			else if (c.n_problems) { if (!pset) { bp0 = c.first; pset = true; } bp1 = (size_t)c.first + c.n_problems; }
-		}
-		const size_t np = bp1 - bp0;
-		uint8_t* trp = nullptr;
-		size_t cap = 0;
-		if (np && env.want_transcript) {
-			for (size_t k = bp0; k < bp1; ++k) cap += (size_t)env.qlen(rw.cprobs[k].query) + (size_t)env.tlen(rw.cprobs[k].target);
-			if (w.tr.resize(ctx, cap)) return 1;
-			trp = w.tr.data();
-		}
-		if (w.cres.resize(ctx, np)) return 1;
-		d.stats.host_bridge_ms += ms_since(t0);
-		t0 = Clock::now();
-		bs.dp_begin(lane);
-		prof.lap("wait for the DP turn");
-		const int dp_rc = np ? dmnd_banded_swipe(ctx, qb, rb, rw.cprobs.data() + bp0, np, DMND_DP_TRACEBACK, w.cres.data(), trp, cap) : 0;
-		dp_guard.armed = false;
-		bs.dp_end(lane);
-		if (dp_rc) return 1;
-		d.stats.dp2_ms += ms_since(t0);
-		d.stats.dp_problems_round1 += np;
-		prof.lap("banded_swipe (lane's problems)");
-		t0 = Clock::now();
-		const size_t nqh = bk1 - bk0;
-		d.nq_hit = nqh;
-		w.qs.resize(nqh);
-		w.hs.resize(bh1 - bh0);
-		w.run([&](int t) {
-			ThreadCtx& tc = w.tc[(size_t)t];
-			tc.reset();
-			for (size_t k = d.block_begin(t), en = d.block_begin(t + 1); k < en; ++k) {
-				QueryState& q = w.qs[k];
-				const dmnd_chain_query& cq = cqa[bk0 + k];
-				if (cq.flags & DMND_CHAIN_HOST) {
-					q.qid = cq.query;
-					Workspace::HitSeg* hsb = w.hs.data() + ((size_t)cq.first - bh0);
-					for (size_t x = 0; x < cq.n_hits; ++x) { hsb[x].h = rw.hv[cq.first + x]; hsb[x].s = rw.segv[cq.first + x]; hsb[x].site = rw.sitev[cq.first + x]; hsb[x].gf = 1; }
-					d.load_hits(q, tc, hsb, hsb + cq.n_hits);
-					d.start(q, tc);
-				}
-				else {
-					d.start_bridged(q, tc, cq, rw.cprobs.data() + cq.first);
-					d.consume_fused(q, tc, rw.cprobs.data() + cq.first, w.cres.data() + ((size_t)cq.first - bp0), trp);
-				}
-			}
-		});
-		for (const ThreadCtx& tc : w.tc) d.stats.targets += tc.n_targets;
-		d.stats.host_bridge_ms += ms_since(t0);
-		prof.lap("consume chained queries (parallel)");
-	}
-	else if (n_shapes == 1) {
-		const int seed_rc = prep_rc ? 1 : dmnd_search_shape_range(ctx, qb, rb, 0, q_begin, q_end, &hits, &d.stats.seed);
-		seed_turn.pass(lane);
-		if (seed_rc || dmnd_block_bias_wait(ctx)) return 1;  // from here on the lane's stream reads the bias (x-drop extension, DP)
-		prof.lap("search_shape");
-		if (bridge) {
-			d.stats.hits = dmnd_hits_count(hits);
-			d.stats.seed_ms = ms_since(t0);
-			t0 = Clock::now();
-			if (dmnd_hits_chain(ctx, qb, rb, hits, sc.raw_ungapped_xdrop, env.band_slow ? 1 : 0, 64, &co)) { dmnd_hits_free(ctx, hits); return 1; }
-			dmnd_hits_free(ctx, hits);
-			nh = (size_t)co.n_host_hits;
-			if (w.cq.resize(ctx, (size_t)co.n_queries) || w.cprobs.resize(ctx, (size_t)co.n_problems) || w.cres.resize(ctx, (size_t)co.n_problems)
-			    || w.hv.resize(ctx, nh) || w.segv.resize(ctx, nh) || w.sitev.resize(ctx, nh))
-				return 1;
-			if (dmnd_hits_chain_fetch(ctx, w.cq.data(), w.cprobs.data(), w.hv.data(), w.segv.data(), w.sitev.data())) return 1;
-			d.stats.host_bridge_ms += ms_since(t0);
-			prof.lap("hits_chain (device bridge)");
-		}
-		else {
-		nh = dmnd_hits_count(hits);
-		if (w.hv.resize(ctx, nh) || w.segv.resize(ctx, nh) || w.sitev.resize(ctx, nh)) { dmnd_hits_free(ctx, hits); return 1; }
-		if (nh && dmnd_hits_download(ctx, hits, w.hv.data(), nh)) { dmnd_hits_free(ctx, hits); return 1; }
-		// ungapped x-drop extension of every seed hit (align/ungapped.cpp:88, dp/ungapped_align.cpp:150-214), batched
-		// ... together with the sequence and local position of every hit (what load_hits would otherwise search for)
-		if (nh && dmnd_hits_xdrop_sites(ctx, qb, rb, hits, sc.raw_ungapped_xdrop, w.segv.data(), w.sitev.data(), nh)) { dmnd_hits_free(ctx, hits); return 1; }
-		dmnd_hits_free(ctx, hits);
+	w.acc_hits.clear(); w.acc_segs.clear(); w.acc_sites.clear(); w.acc_gf.clear(); w.gfv.clear();
+	for (int sid = 0; sid < n_shapes; ++sid) {
+		HitsGuard hits(d.ctx);
+		dmnd_stage_counters cn;
+		if (dmnd_search_shape_range(d.ctx, d.qb, d.rb, sid, q_begin, q_end, &hits.h, &cn)) return 1;
+		if (n_shapes == 1) turn.pass(lane);  // (with several shapes the turn passes once every shape's hits are down)
+		add_counters(d.stats.seed, cn);
+		const size_t n = dmnd_hits_count(hits.h);
+		std::vector<uint8_t>& gf = n_shapes == 1 ? w.gfv : w.acc_gf;  // this shape's gapped-filter verdicts go to its end
+		gf.resize(gf.size() + n, 1);
+		if (w.hv.resize(d.ctx, n) || w.segv.resize(d.ctx, n) || w.sitev.resize(d.ctx, n)) return 1;
+		if (n && (dmnd_hits_download(d.ctx, hits.h, w.hv.data(), n) || dmnd_hits_xdrop_sites(d.ctx, d.qb, d.rb, hits.h, env.sc->raw_ungapped_xdrop, w.segv.data(), w.sitev.data(), n)))
+			return 1;
+		if (n && env.gapped_filter && dmnd_hits_gapped_filter(d.ctx, d.qb, d.rb, hits.h, gf.data() + gf.size() - n, n)) return 1;  // align/gapped_filter.cpp, per hit
+		if (n_shapes > 1) {
+			w.acc_hits.insert(w.acc_hits.end(), w.hv.begin(), w.hv.end()); w.acc_segs.insert(w.acc_segs.end(), w.segv.begin(), w.segv.end());
+			w.acc_sites.insert(w.acc_sites.end(), w.sitev.begin(), w.sitev.end());
 		}
 	}
-	else {
-		// run_ref_chunk's loop over the shapes (run/double_indexed.cpp:185-214): SEED_MASK bits set by one shape stay visible
-		// to the next ones, the hits of all shapes feed one extension; every shape's hits arrive grouped by query and are merged
-		// into one query-grouped list (counting sort by query, stable)
-		int rc = prep_rc || dmnd_block_bias_wait(ctx);  // (the x-drop extension and the gapped filter of every shape read the bias)
-		std::vector<dmnd_hit>& ah = w.acc_hits; std::vector<dmnd_segment>& as = w.acc_segs; std::vector<dmnd_hit_site>& at = w.acc_sites;
-		ah.clear(); as.clear(); at.clear(); w.acc_gf.clear();
-		for (int sid = 0; sid < n_shapes && !rc; ++sid) {
-			dmnd_stage_counters cn;
-			rc = dmnd_search_shape_range(ctx, qb, rb, sid, q_begin, q_end, &hits, &cn);
-			if (rc) break;
-			d.stats.seed.seeds_hit += cn.seeds_hit; d.stats.seed.seed_hits += cn.seed_hits; d.stats.seed.tentative_matches1 += cn.tentative_matches1;
-			d.stats.seed.tentative_matches2 += cn.tentative_matches2; d.stats.seed.tentative_matches3 += cn.tentative_matches3; d.stats.seed.masked_seeds += cn.masked_seeds;
-			const size_t n = dmnd_hits_count(hits);
-			if (w.hv.resize(ctx, n) || w.segv.resize(ctx, n) || w.sitev.resize(ctx, n)) rc = 1;
-			if (!rc && n) rc = dmnd_hits_download(ctx, hits, w.hv.data(), n) || dmnd_hits_xdrop_sites(ctx, qb, rb, hits, sc.raw_ungapped_xdrop, w.segv.data(), w.sitev.data(), n);
-			w.gf_tmp.assign(n, 1);
-			if (!rc && n && env.gapped_filter) rc = dmnd_hits_gapped_filter(ctx, qb, rb, hits, w.gf_tmp.data(), n);  // align/gapped_filter.cpp, per hit
-			dmnd_hits_free(ctx, hits);
-			if (!rc) { ah.insert(ah.end(), w.hv.begin(), w.hv.end()); as.insert(as.end(), w.segv.begin(), w.segv.end()); at.insert(at.end(), w.sitev.begin(), w.sitev.end());
-			           w.acc_gf.insert(w.acc_gf.end(), w.gf_tmp.begin(), w.gf_tmp.end()); }
-		}
-		seed_turn.pass(lane);
-		if (rc) return 1;
-		prof.lap("search_shape (all shapes)");
+	turn.pass(lane);
+	prof.lap("search_shape + hits download (every shape)");
+	nh = w.hv.size();
+	if (n_shapes > 1) {
+		const std::vector<dmnd_hit>& ah = w.acc_hits;
 		nh = ah.size();
-		if (w.hv.resize(ctx, nh) || w.segv.resize(ctx, nh) || w.sitev.resize(ctx, nh)) return 1;
+		if (w.hv.resize(d.ctx, nh) || w.segv.resize(d.ctx, nh) || w.sitev.resize(d.ctx, nh)) return 1;
 		std::vector<size_t> off((size_t)(q_end - q_begin) + 1, 0);
 		for (const dmnd_hit& h : ah) ++off[(size_t)(h.query - q_begin) + 1];
 		for (size_t k = 1; k < off.size(); ++k) off[k] += off[k - 1];
 		w.gfv.resize(nh);
-		for (size_t k = 0; k < nh; ++k) { const size_t o = off[(size_t)(ah[k].query - q_begin)]++; w.hv[o] = ah[k]; w.segv[o] = as[k]; w.sitev[o] = at[k]; w.gfv[o] = w.acc_gf[k]; }
+		for (size_t k = 0; k < nh; ++k) {
+			const size_t o = off[(size_t)(ah[k].query - q_begin)]++;
+			w.hv[o] = ah[k]; w.segv[o] = w.acc_segs[k]; w.sitev[o] = w.acc_sites[k]; w.gfv[o] = w.acc_gf[k];
+		}
 	}
-	const bool block_mode = bs.on && bridge;
-	if (n_shapes == 1) w.gfv.assign(nh, 1);
-	if (env.min_length_ratio > 0.0 && !bridge) {
+	if (env.min_length_ratio > 0.0) {
 		// mutual-coverage seed stage (search/hamming/kernel_mutual_cov.h:28-52, chosen by stage1_dispatch when min_length_ratio > 0): over
 		// length-sorted blocks its two cursors admit exactly the (query, target) pairs with qlen / tlen >= mlr and tlen / qlen >= mlr.
 		// Every later step of the seed stage is per pair, so dropping the other pairs' hits here gives the same hit list.
@@ -1404,73 +1308,79 @@ static int lane_run(dmnd_ctx* ctx, dmnd_block* qb, const dmnd_block* rb, const E
 		}
 		nh = o;
 	}
-	if (!block_mode && dmnd_block_clear_seed_mask_range(ctx, qb, q_begin, q_end)) return 1;  // run/double_indexed.cpp:211-212
-	prof.lap("hits download");
-	if (!bridge) { d.stats.seed_ms = ms_since(t0); d.stats.hits = nh; }
-	const int T = host_threads;
-	const uint32_t C = env.contexts;
+	d.stats.hits = nh;
+	return 0;
+}
 
-	if (block_mode) {}  // (its queries were consumed above)
-	else if (bridge) {
-		// ---- the device-chained problem list is aligned where it lies; the host then only scores and culls (consume_fused)
-		t0 = Clock::now();
-		const size_t np = (size_t)co.n_problems, nqh = (size_t)co.n_queries;
-		uint8_t* trp = nullptr;
-		size_t cap = 0;
-		if (np && env.want_transcript) {
-			std::vector<size_t> part((size_t)T, 0);
-			w.run([&](int t) {
-				size_t c = 0;
-				for (size_t k = np * (size_t)t / (size_t)T, en = np * (size_t)(t + 1) / (size_t)T; k < en; ++k) c += (size_t)env.qlen(w.cprobs[k].query) + (size_t)env.tlen(w.cprobs[k].target);
-				part[(size_t)t] = c;
-			});
-			for (size_t c : part) cap += c;
-			if (w.tr.resize(ctx, cap)) return 1;
-			trp = w.tr.data();
-		}
-		if (np && dmnd_banded_swipe_chained(ctx, qb, rb, np, DMND_DP_TRACEBACK, w.cres.data(), trp, cap)) return 1;
-		d.stats.dp2_ms += ms_since(t0);
-		d.stats.dp_problems_round1 += np;
-		prof.lap("banded_swipe (chained list)");
-		t0 = Clock::now();
-		d.nq_hit = nqh;
-		w.qs.resize(nqh);
-		w.hs.resize(nh);
-		std::atomic<int> bad(0);
+// Bridged mode: the device-chained problem list is aligned where it lies and the host only scores and culls (consume_fused); the
+// queries the device code left to the host load their hits as on the host path.
+static int load_bridged(Driver& d, const dmnd_chain_out& co, Prof& prof) {
+	Workspace& w = *d.ws;
+	const Env& env = d.env;
+	const size_t T = (size_t)d.T;
+	auto t0 = Clock::now();
+	const size_t np = (size_t)co.n_problems, nqh = (size_t)co.n_queries;
+	uint8_t* trp = nullptr;
+	size_t cap = 0;
+	if (np && env.want_transcript) {
+		std::vector<size_t> part(T, 0);
 		w.run([&](int t) {
-			ThreadCtx& tc = w.tc[(size_t)t];
-			tc.reset();
-			for (size_t k = d.block_begin(t), en = d.block_begin(t + 1); k < en; ++k) {
-				QueryState& q = w.qs[k];
-				const dmnd_chain_query& cq = w.cq[k];
-				if (k > 0 && cq.query <= w.cq[k - 1].query) bad = 1;
-				if (cq.flags & DMND_CHAIN_HOST) {
-					q.qid = cq.query;
-					for (size_t x = cq.first; x < (size_t)cq.first + cq.n_hits; ++x) { w.hs[x].h = w.hv[x]; w.hs[x].s = w.segv[x]; w.hs[x].site = w.sitev[x]; w.hs[x].gf = 1; }
-					d.load_hits(q, tc, w.hs.data() + cq.first, w.hs.data() + cq.first + cq.n_hits);
-					d.start(q, tc);
-				}
-				else {
-					d.start_bridged(q, tc, cq, w.cprobs.data() + cq.first);
-					d.consume_fused(q, tc, w.cprobs.data() + cq.first, w.cres.data() + cq.first, trp);
-				}
-			}
+			const size_t b = np * (size_t)t / T, e = np * (size_t)(t + 1) / T;
+			part[(size_t)t] = transcript_cap(env, w.cprobs.data() + b, e - b);
 		});
-		if (bad) { dmnd_set_last_error("dmnd_blastp: dmnd_hits_chain records not in ascending query order"); return 1; }
-		for (const ThreadCtx& tc : w.tc) d.stats.targets += tc.n_targets;
-		d.stats.host_bridge_ms += ms_since(t0);
-		prof.lap("consume chained queries (parallel)");
+		for (size_t c : part) cap += c;
+		if (w.tr.resize(d.ctx, cap)) return 1;
+		trp = w.tr.data();
 	}
-	else {
-	// ---- group by query (hits arrive grouped by ascending query id): boundaries found in parallel
+	if (np && dmnd_banded_swipe_chained(d.ctx, d.qb, d.rb, np, DMND_DP_TRACEBACK, w.cres.data(), trp, cap)) return 1;
+	d.stats.dp2_ms += ms_since(t0);
+	d.stats.dp_problems_round1 += np;
+	prof.lap("banded_swipe (chained list)");
 	t0 = Clock::now();
-	std::vector<std::vector<size_t>> tl_bounds((size_t)T);
+	d.nq_hit = nqh;
+	w.qs.resize(nqh);
+	w.hs.resize((size_t)co.n_host_hits);
+	std::atomic<int> bad(0);
+	w.run([&](int t) {
+		ThreadCtx& tc = w.tc[(size_t)t];
+		tc.reset();
+		for (size_t k = d.block_begin(t), en = d.block_begin(t + 1); k < en; ++k) {
+			QueryState& q = w.qs[k];
+			const dmnd_chain_query& cq = w.cq[k];
+			if (k > 0 && cq.query <= w.cq[k - 1].query) bad = 1;
+			if (cq.flags & DMND_CHAIN_HOST) {
+				q.qid = cq.query;
+				Workspace::HitSeg* hs = w.gather(cq.first, (size_t)cq.first + cq.n_hits);
+				d.load_hits(q, tc, hs, hs + cq.n_hits);
+				d.start(q, tc);
+			}
+			else {
+				d.start_bridged(q, tc, cq, w.cprobs.data() + cq.first);
+				d.consume_fused(q, tc, w.cprobs.data() + cq.first, w.cres.data() + cq.first, trp);
+			}
+		}
+	});
+	if (bad) { dmnd_set_last_error("dmnd_blastp: dmnd_hits_chain records not in ascending query order"); return 1; }
+	d.stats.host_bridge_ms += ms_since(t0);
+	prof.lap("consume chained queries (parallel)");
+	return 0;
+}
+
+// Host path: hv [0, nh) is grouped by ascending query id; one group per query = all its contexts (search/hit.h:71-78), boundaries found
+// in parallel.  Every query then loads its hits (load_hits + start, or legacy_init in frameshift mode).
+static int load_host(Driver& d, size_t nh, Prof& prof) {
+	Workspace& w = *d.ws;
+	const Env& env = d.env;
+	const size_t T = (size_t)d.T;
+	const uint32_t C = env.contexts;
+	auto t0 = Clock::now();
+	std::vector<std::vector<size_t>> tl_bounds(T);
 	std::atomic<int> bad(0);
 	w.run([&](int t) {
 		auto& v = tl_bounds[(size_t)t];
 		v.clear();
-		for (size_t i = nh * (size_t)t / (size_t)T, en = nh * (size_t)(t + 1) / (size_t)T; i < en; ++i)
-			if (i == 0 || w.hv[i].query / C != w.hv[i - 1].query / C) {  // one group per query = all its contexts (search/hit.h:71-78)
+		for (size_t i = nh * (size_t)t / T, en = nh * (size_t)(t + 1) / T; i < en; ++i)
+			if (i == 0 || w.hv[i].query / C != w.hv[i - 1].query / C) {
 				if (i > 0 && w.hv[i].query < w.hv[i - 1].query) bad = 1;
 				v.push_back(i);
 			}
@@ -1491,23 +1401,26 @@ static int lane_run(dmnd_ctx* ctx, dmnd_block* qb, const dmnd_block* rb, const E
 		for (size_t k = d.block_begin(t), en = d.block_begin(t + 1); k < en; ++k) {
 			QueryState& q = w.qs[k];
 			q.qid = w.hv[w.qstart[k]].query / C * C;
-			for (size_t x = w.qstart[k]; x < w.qstart[k + 1]; ++x) { w.hs[x].h = w.hv[x]; w.hs[x].s = w.segv[x]; w.hs[x].site = w.sitev[x]; w.hs[x].gf = w.gfv[x]; }
-			if (env.frame_shift) { d.legacy_init(k, q, tc, w.hs.data() + w.qstart[k], w.hs.data() + w.qstart[k + 1]); continue; }
-			d.load_hits(q, tc, w.hs.data() + w.qstart[k], w.hs.data() + w.qstart[k + 1]);
+			Workspace::HitSeg* hs = w.gather(w.qstart[k], w.qstart[k + 1]);
+			Workspace::HitSeg* he = hs + (w.qstart[k + 1] - w.qstart[k]);
+			if (env.frame_shift) { d.legacy_init(k, q, tc, hs, he); continue; }
+			d.load_hits(q, tc, hs, he);
 			d.start(q, tc);
 		}
 	});
-	for (const ThreadCtx& tc : w.tc) d.stats.targets += tc.n_targets;
 	d.stats.host_bridge_ms += ms_since(t0);
 	prof.lap("load_hits (parallel)");
-	}
+	return 0;
+}
 
-	if (env.frame_shift ? d.run_legacy() : d.run_waves()) return 1;
-	prof.lap("run_waves");
-
-	// ---- emit: per-thread counts -> offsets -> parallel fill (matches grouped by ascending query)
-	t0 = Clock::now();
-	std::vector<size_t> moff((size_t)T + 1, 0), troff((size_t)T + 1, 0);
+// Emit: per-thread counts -> offsets -> parallel fill of the lane's output (matches grouped by ascending query), with the counters the
+// threads kept.
+static void emit_matches(Driver& d, LaneOut& lo, Prof& prof) {
+	Workspace& w = *d.ws;
+	const Scoring& sc = *d.env.sc;
+	const size_t T = (size_t)d.T;
+	auto t0 = Clock::now();
+	std::vector<size_t> moff(T + 1, 0), troff(T + 1, 0);
 	w.run([&](int t) {
 		ThreadCtx& tc = w.tc[(size_t)t];
 		for (size_t k = d.block_begin(t), en = d.block_begin(t + 1); k < en; ++k) {
@@ -1516,17 +1429,18 @@ static int lane_run(dmnd_ctx* ctx, dmnd_block* qb, const dmnd_block* rb, const E
 			else tc.unaligned.push_back(w.qs[k].qid);
 		}
 	});
-	for (int t = 0; t < T; ++t) {
-		moff[(size_t)t + 1] = moff[(size_t)t] + w.tc[(size_t)t].n_matches;
-		troff[(size_t)t + 1] = troff[(size_t)t] + w.tc[(size_t)t].trbuf.size();
-		d.stats.queries_aligned += w.tc[(size_t)t].n_aligned;
-		d.stats.cells_round1 += w.tc[(size_t)t].cells1; d.stats.cells_round2 += w.tc[(size_t)t].cells2;
-		d.stats.dp_problems_round2 += w.tc[(size_t)t].fused_r2; d.stats.dp_problems_fused += w.tc[(size_t)t].fused_r1;
-		d.stats.targets_extended += w.tc[(size_t)t].n_extended;
-		lo.unaligned.insert(lo.unaligned.end(), w.tc[(size_t)t].unaligned.begin(), w.tc[(size_t)t].unaligned.end());  // threads own ascending query ranges
+	for (size_t t = 0; t < T; ++t) {
+		const ThreadCtx& tc = w.tc[t];
+		moff[t + 1] = moff[t] + tc.n_matches;
+		troff[t + 1] = troff[t] + tc.trbuf.size();
+		d.stats.targets += tc.n_targets; d.stats.queries_aligned += tc.n_aligned;
+		d.stats.cells_round1 += tc.cells1; d.stats.cells_round2 += tc.cells2;
+		d.stats.dp_problems_round2 += tc.fused_r2; d.stats.dp_problems_fused += tc.fused_r1;
+		d.stats.targets_extended += tc.n_extended;
+		lo.unaligned.insert(lo.unaligned.end(), tc.unaligned.begin(), tc.unaligned.end());  // threads own ascending query ranges
 	}
-	lo.matches->resize(moff[(size_t)T]);
-	lo.transcripts->resize(troff[(size_t)T]);
+	lo.matches->resize(moff[T]);
+	lo.transcripts->resize(troff[T]);
 	w.run([&](int t) {
 		const ThreadCtx& tc = w.tc[(size_t)t];
 		dmnd_match* o = lo.matches->data() + moff[(size_t)t];
@@ -1549,21 +1463,43 @@ static int lane_run(dmnd_ctx* ctx, dmnd_block* qb, const dmnd_block* rb, const E
 	d.stats.matches = lo.matches->size();
 	d.stats.host_bridge_ms += ms_since(t0);
 	prof.lap("emit matches");
+}
+
+// The stages of one lane.  Wall time up to the end of the seed stage is seed_ms (the bridged mode's seed stage ends with its search),
+// the DP calls go to dp1_ms / dp2_ms, and the host work between them (dmnd_hits_chain included) to host_bridge_ms.
+static int lane_run(dmnd_ctx* ctx, dmnd_block* qb, const dmnd_block* rb, const Env& env, uint32_t q_begin, uint32_t q_end,
+                    Workspace& w, int host_threads, LaneOut& lo, int lane, SeedTurn& turn) {
+	TurnRelease release{ turn, lane };
+	auto t_total = Clock::now();
+	Driver d;
+	d.ctx = ctx; d.qb = qb; d.rb = rb; d.ws = &w; d.T = host_threads; d.env = env;
+	std::memset(&d.stats, 0, sizeof d.stats);
+	w.lane = lane;
+	dmnd_timing tm0, tm1;
+	dmnd_timing_fetch(ctx, &tm0, DMND_TIMING_THIS_CONTEXT);  // snapshot: the device counters of this call are reported as a delta
+	Prof prof;
+	prof.lane = lane;
+	const auto t_seed = Clock::now();
+	if (prepare_range(d, q_begin, q_end, lane, turn, prof)) return 1;
+	dmnd_chain_out co{};
+	size_t nh = 0;
+	if (env.bridge ? seed_bridged(d, q_begin, q_end, lane, turn, t_seed, co, prof) : seed_host(d, q_begin, q_end, lane, turn, nh, prof)) return 1;
+	if (dmnd_block_clear_seed_mask_range(ctx, qb, q_begin, q_end)) return 1;  // run/double_indexed.cpp:211-212
+	prof.lap("clear seed mask");
+	if (!env.bridge) d.stats.seed_ms = ms_since(t_seed);
+	if (env.bridge ? load_bridged(d, co, prof) : load_host(d, nh, prof)) return 1;
+	if (env.frame_shift ? d.run_legacy() : d.run_waves()) return 1;
+	prof.lap("run_waves");
+	emit_matches(d, lo, prof);
 	d.stats.total_ms = ms_since(t_total);
-	{
-		dmnd_timing tm1; dmnd_timing_fetch(ctx, &tm1, DMND_TIMING_THIS_CONTEXT);
-		dmnd_timing& dv = d.stats.device;
-		dv.seed_ms = tm1.seed_ms - tm0.seed_ms; dv.dp_score_ms = tm1.dp_score_ms - tm0.dp_score_ms; dv.dp_trace_ms = tm1.dp_trace_ms - tm0.dp_trace_ms;
-		dv.h2d_ms = tm1.h2d_ms - tm0.h2d_ms; dv.d2h_ms = tm1.d2h_ms - tm0.d2h_ms;
-		dv.launches = tm1.launches - tm0.launches; dv.h2d_bytes = tm1.h2d_bytes - tm0.h2d_bytes; dv.d2h_bytes = tm1.d2h_bytes - tm0.d2h_bytes;
-	}
+	dmnd_timing_fetch(ctx, &tm1, DMND_TIMING_THIS_CONTEXT);
+	d.stats.device = device_delta(tm1, tm0);
 	lo.stats = d.stats;
 	return 0;
 }
 
 static void add_stats(dmnd_run_stats& a, const dmnd_run_stats& b) {
-	a.seed.seeds_hit += b.seed.seeds_hit; a.seed.seed_hits += b.seed.seed_hits; a.seed.tentative_matches1 += b.seed.tentative_matches1;
-	a.seed.tentative_matches2 += b.seed.tentative_matches2; a.seed.tentative_matches3 += b.seed.tentative_matches3; a.seed.masked_seeds += b.seed.masked_seeds;
+	add_counters(a.seed, b.seed);
 	a.hits += b.hits; a.targets += b.targets; a.dp_problems_round1 += b.dp_problems_round1; a.dp_problems_round2 += b.dp_problems_round2;
 	a.cells_round1 += b.cells_round1; a.cells_round2 += b.cells_round2; a.queries_aligned += b.queries_aligned; a.matches += b.matches;
 	a.dp_problems_fused += b.dp_problems_fused; a.targets_extended += b.targets_extended;
@@ -1679,6 +1615,7 @@ static int blastp_impl(dmnd_ctx* ctx, dmnd_block* qb, const dmnd_block* rb, cons
 		e.n_shapes = mt->n_shapes; e.gapped_filter = mt->gapped_filter_evalue > 0.0; e.band_slow = opts->ext_mode == 0 ? mt->band_slow : opts->ext_mode == 2; e.ranking_letters = mt->ranking_letters;  // --ext (search/setup.cpp:377-384)
 		if (e.frame_shift) e.gapped_filter = false;  // Extension::gapped_filter belongs to Extension::extend, which frameshift mode does not run
 	}
+	e.bridge = e.n_shapes == 1 && e.fuse && e.contexts == 1 && !e.gapped_filter && !e.frame_shift;
 	if (mask_algo) {
 		// "Masking reference" (run/double_indexed.cpp:122-127) and the reference block's motif table, before its seed index
 		uint64_t n_hard = 0;
@@ -1705,17 +1642,13 @@ static int blastp_impl(dmnd_ctx* ctx, dmnd_block* qb, const dmnd_block* rb, cons
 		if (dmnd_ctx_lane(ctx, l - 1, &lctx[(size_t)l])) return 1;
 	SeedTurn seed_turn;
 	seed_turn.masked.assign((size_t)nlanes, 0);
-	BlockStage bs;
-	bs.nlanes = nlanes;
-	bs.on = nlanes > 1 && e.n_shapes == 1 && e.fuse && e.contexts == 1 && !e.gapped_filter && !e.frame_shift && std::getenv("DMND_HOST_BRIDGE") == nullptr
-	        && std::getenv("DMND_PIPELINE_BLOCK") != nullptr;  // opt-in: measured slower than the per-lane pipeline (see BlockStage)
 	auto body = [&](int l) {
 		LaneOut& o = lo[(size_t)l];
 		try {
-			o.rc = lane_run(lctx[(size_t)l], qb, rb, e, sc, cut[(size_t)l], cut[(size_t)l + 1], *sh.lanes[(size_t)l], host_threads, o, l, seed_turn, bs);
+			o.rc = lane_run(lctx[(size_t)l], qb, rb, e, cut[(size_t)l], cut[(size_t)l + 1], *sh.lanes[(size_t)l], host_threads, o, l, seed_turn);
 			if (o.rc) o.error = dmnd_last_error();  // the error text is thread-local in the CUDA library
 		}
-		catch (const std::exception& ex) { o.rc = 1; o.error = std::string("dmnd_blastp: ") + ex.what(); seed_turn.set_masked(l); seed_turn.pass(l); bs.abort(); }
+		catch (const std::exception& ex) { o.rc = 1; o.error = std::string("dmnd_blastp: ") + ex.what(); }
 	};
 	std::vector<std::thread> th;
 	for (int l = 1; l < nlanes; ++l) th.emplace_back(body, l);

@@ -169,13 +169,8 @@ int dmnd_block_build_index(dmnd_ctx* ctx, dmnd_block* b, int sid);
 /* Fills the block's bias array on the device: mode 1 = HauserCorrection of every sequence (stats/hauser_correction.cpp:
  * 53-109, window 40, fp32, rounded half away from zero), mode 0 = zeros (--comp-based-stats 0). */
 int dmnd_block_compute_bias(dmnd_ctx* ctx, dmnd_block* b, int mode);
-/* Same for the sequences [s_begin, s_end) only, on `ctx`'s stream (a lane computes the bias of its own query range). */
+/* Same for the sequences [s_begin, s_end) only, on `ctx`'s stream (a lane computes the bias of its own query range); complete on return. */
 int dmnd_block_compute_bias_range(dmnd_ctx* ctx, dmnd_block* b, int mode, uint32_t s_begin, uint32_t s_end);
-/* Same, without waiting: the work is queued on the context's second stream behind everything `ctx` has issued so far (masking of the
- * range) and runs beside what `ctx` issues next -- the seed stage reads letters only.  dmnd_block_bias_wait(ctx) makes the context's
- * stream wait for it (no host wait); call it before the first consumer of the bias (x-drop extension, banded swipe). */
-int dmnd_block_compute_bias_range_async(dmnd_ctx* ctx, dmnd_block* b, int mode, uint32_t s_begin, uint32_t s_end);
-int dmnd_block_bias_wait(dmnd_ctx* ctx);
 /* Reads back the block's bias array. */
 int dmnd_block_download_bias(dmnd_ctx* ctx, const dmnd_block* b, int8_t* bias, size_t raw_len);
 /* Same, on the library's copy stream: returns at once, dmnd_copy_wait() blocks until `bias` is complete.  Overlaps with

@@ -174,8 +174,6 @@ int dmnd_block_compute_bias_range(dmnd_ctx* ctx, dmnd_block* b, int mode, uint32
 	}
 	return 0;
 }
-int dmnd_block_compute_bias_range_async(dmnd_ctx* ctx, dmnd_block* b, int mode, uint32_t s_begin, uint32_t s_end) { return dmnd_block_compute_bias_range(ctx, b, mode, s_begin, s_end); }
-int dmnd_block_bias_wait(dmnd_ctx* ctx) { (void)ctx; return 0; }
 int dmnd_block_compute_bias(dmnd_ctx* ctx, dmnd_block* b, int mode) {
 	if (mode != 0 && mode != 1) return fail("dmnd_block_compute_bias: unknown mode");
 	memset(b->bias, 0, b->raw_len);

@@ -46,14 +46,14 @@ def test_live_reference_run(oracle_lib, seed):
     assert text_digest(api.fmt6(m)) == gold
 
 
-@pytest.mark.parametrize("lanes", ["1", "3", "3-block"])
+@pytest.mark.parametrize("lanes", ["1", "3", "3-nofuse"])
 def test_query_lanes_do_not_change_results(oracle_lib, lanes, monkeypatch):
-    """The P layer may split the query block into lanes that run concurrently: output must be independent of it.  "3-block" = the
-    opt-in block mode (DMND_PIPELINE_BLOCK: one seed stage + one dmnd_hits_chain for the whole block, DP and host work per lane range)."""
+    """The P layer may split the query block into lanes that run concurrently: output must be independent of it.  "3-nofuse" =
+    DMND_NO_FUSE, which also turns the device bridge off: single-shape blastp then takes the host path in every lane."""
     from diamond_b200 import api
     monkeypatch.setenv("DMND_LANES", lanes[0])
-    if lanes.endswith("block"):
-        monkeypatch.setenv("DMND_PIPELINE_BLOCK", "1")
+    if lanes.endswith("nofuse"):
+        monkeypatch.setenv("DMND_NO_FUSE", "1")
     w, q_raw, q_lim, r_raw, r_lim = workload_blocks("fam2")
     ctx = api.Context(oracle_lib, threads=8, comp_based_stats=1, want_transcript=True)
     m, tr, st = ctx.blastp(q_raw, q_lim, r_raw, r_lim)
